@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- V'DJer de Bruijn graph build+prune throughput on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload NAME] [--dump-outputs DIR]
 
 A step = one graph build (estimate -> pass 1 -> prune -> pass 2 -> export) over the whole
 synthetic read set.  Unit: windows (k-mer positions) per second, W = records * (L-k+1).
@@ -42,6 +42,8 @@ METRIC = "graph_build_prune_windows_per_sec"
 UNIT = "windows/s"
 DEFAULT_WORKLOAD = "igh_2x50_5M"  # BASELINE.json configs[1]
 NCU_SUMMARY = "profiles/ncu_r2_summary.json"
+GRAPH_ARRAYS = ["first_pos", "frequency", "out_deg", "in_deg", "out_succ", "in_pred"]
+DUMP_BYTES = 64_000_000   # --dump-outputs writes less than this in all
 
 
 def peaks():
@@ -197,7 +199,26 @@ def cpu_baseline(wl: dict, sample_pairs: int, extras: bool = False):
         except Exception as e:   # the -g library is optional
             out["reference_flags_g"] = {"unavailable": str(e)[:100]}
     out["_primary"], out["_secondary"] = primary, secondary
+    out["_graph"] = r
     return out
+
+
+def dump_outputs(out_dir: str, graph) -> dict:
+    """--dump-outputs: the graph the caller of the timed path received in the last step (node rows in
+    creation order, as vdjgraph_fetch returns them) as DIR/<array>.npy in float64, so that two builds
+    can be compared output for output.  Every value is an integer below 2^53, so float64 holds it
+    exactly.  A graph too large for DUMP_BYTES is sampled: node_index.npy holds the rows kept, a
+    seeded choice that depends only on the node count; n_nodes.npy holds the count."""
+    arrays = {n: (graph[n] if isinstance(graph, dict) else getattr(graph, n)) for n in GRAPH_ARRAYS}
+    n = len(arrays["first_pos"])
+    row_bytes = 8 * (1 + sum(int(np.prod(a.shape[1:])) for a in arrays.values()))   # + node_index
+    rows = min(n, (DUMP_BYTES - 4096) // row_bytes)                                   # 4096: .npy headers
+    index = np.arange(n) if rows == n else np.sort(np.random.default_rng(0).choice(n, rows, replace=False))
+    out = {"n_nodes": np.array([n]), "node_index": index, **{name: a[index] for name, a in arrays.items()}}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float64))
+    return {"dir": out_dir, "nodes": n, "rows": rows, "dtype": "float64"}
 
 
 def run_reference(args, wl, rank):
@@ -220,6 +241,8 @@ def run_reference(args, wl, rank):
             "cpu_baseline": {k: v for k, v in cb.items() if not k.startswith("_")},
             "e2e": {"value": value, "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}}
     line["cpu_baseline"]["value"] = value
+    if args.dump_outputs:
+        line["outputs_dumped"] = dump_outputs(args.dump_outputs, cb["_graph"])
     print(json.dumps(line), flush=True)
 
 
@@ -385,7 +408,12 @@ def main():
     ap.add_argument("--rounds", type=int, default=0, help="rounds over groups of hash units (0 = auto: 1 unless the working set exceeds HBM)")
     ap.add_argument("--cpu-sample-pairs", type=int, default=1_000_000)
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the graph of the last step as DIR/<array>.npy (float64; "
+                         "a fixed, seeded sample of the nodes when it exceeds 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     from vdjer_b200 import synth
     wl = dict(synth.CONFIGS[args.workload])
@@ -465,6 +493,8 @@ def main():
     barrier()
     wall_dev = (time.perf_counter() - t0) / args.steps
     clocks = sampler.stop()
+    # the graph of the last timed step (rank 0), copied out before the checks below restage the builder
+    last_graph = (db.fetch() if sharded else gb.fetch()) if args.dump_outputs else None
     stats = per_kernel[-1]
     phase_ms = dict(db.phase_ms) if sharded else None
     W = stats["n_windows"]
@@ -650,6 +680,8 @@ def main():
                     line["cpu_baseline"]["glue_rebuild"] = gr
                     if "ms_at_this_graph" in gr:
                         line["e2e"]["ms_with_glue_rebuild"] = gr["e2e_ms_with_layout"] + gr["ms_at_this_graph"]
+        if last_graph is not None:
+            line["outputs_dumped"] = dump_outputs(args.dump_outputs, last_graph)
         print(json.dumps(line), flush=True)
     if world > 1:
         db.close()
