@@ -60,6 +60,8 @@ double wall_ms() {
     return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now().time_since_epoch()).count();
 }
 
+/* DevBuf and PinBuf own their allocation: it is freed when they are destroyed.  They move (a growing
+ * std::vector<StageWorker> moves its workers' buffers) but do not copy, which would free twice. */
 struct DevBuf {
     void *p = nullptr;
     size_t cap = 0;
@@ -67,6 +69,11 @@ struct DevBuf {
      * have the old allocation mapped.  It is parked here until vdjgraph_shard_release_retired(). */
     bool exported = false;
     std::vector<void *> retired;
+    DevBuf() = default;
+    DevBuf(DevBuf &&o) noexcept : p(o.p), cap(o.cap), exported(o.exported), retired(std::move(o.retired)) { o.p = nullptr; o.cap = 0; }
+    DevBuf(const DevBuf &) = delete;
+    DevBuf &operator=(const DevBuf &) = delete;
+    ~DevBuf() { release(); }
     int ensure(size_t bytes) {
         if (bytes <= cap) return 0;
         if (p) { if (exported) retired.push_back(p); else cudaFree(p); }
@@ -106,6 +113,11 @@ struct DevBuf {
 struct PinBuf {
     void *p = nullptr;
     size_t cap = 0;
+    PinBuf() = default;
+    PinBuf(PinBuf &&o) noexcept : p(o.p), cap(o.cap) { o.p = nullptr; o.cap = 0; }
+    PinBuf(const PinBuf &) = delete;
+    PinBuf &operator=(const PinBuf &) = delete;
+    ~PinBuf() { release(); }
     int ensure(size_t bytes) {
         if (bytes <= cap) return 0;
         if (p) cudaFreeHost(p);
@@ -130,9 +142,67 @@ struct StageWorker {
     cudaStream_t stream = nullptr;
     PinBuf buf[2];
     DevBuf dbuf[2];
-    cudaEvent_t ev[2] = { nullptr, nullptr };
+    cudaEvent_t done[2] = { nullptr, nullptr };   /* recorded behind the chunk that buffer b holds */
     bool busy[2] = { false, false };
 };
+
+/* the nodes' k-mers are exported: asked for, or hashed by the hash-map layout */
+bool want_keys(uint32_t flags) { return flags & (VDJGRAPH_FLAG_EXPORT_KEYS | VDJGRAPH_FLAG_HASHMAP_LAYOUT); }
+
+/* The graph's node arrays on the device (k_export / k_unpack_* write them) and their page-locked host
+ * mirrors (vdjgraph_fetch).  kmer_lo and kmer_hi are last: they exist only when keys are wanted. */
+struct NodeArrays {
+    enum { FIRST_POS, FREQUENCY, OUT_DEG, IN_DEG, OUT_SUCC, IN_PRED, KMER_LO, KMER_HI, N };
+    static constexpr size_t elem_bytes[N] = { 8, 2, 1, 1, 16, 16, 8, 8 };
+    DevBuf d[N];
+    PinBuf h[N];
+    static int count(bool keys) { return keys ? N : KMER_LO; }
+    int ensure(uint64_t n, bool keys) {
+        for (int i = 0; i < count(keys); i++)
+            if (int rc = d[i].ensure(std::max<uint64_t>(n, 1) * elem_bytes[i])) return rc;
+        return 0;
+    }
+    /* k_export / k_unpack_* arguments that write into these arrays (the other fields zero) */
+    ExportArgs export_args(bool keys) const {
+        ExportArgs a{};
+        a.first_pos = d[FIRST_POS].as<u64>(); a.frequency = d[FREQUENCY].as<u16>();
+        a.out_deg = d[OUT_DEG].as<u8>(); a.in_deg = d[IN_DEG].as<u8>();
+        a.out_succ = d[OUT_SUCC].as<u32>(); a.in_pred = d[IN_PRED].as<u32>();
+        a.kmer_lo = keys ? d[KMER_LO].as<u64>() : nullptr; a.kmer_hi = keys ? d[KMER_HI].as<u64>() : nullptr;
+        return a;
+    }
+    /* the first n nodes to the host mirrors (s is synchronised) and r's arrays pointed at them; adds the bytes copied to `bytes` */
+    int fetch(uint64_t n, bool keys, cudaStream_t s, vdjgraph_result &r, uint64_t &bytes) {
+        for (int i = 0; i < count(keys); i++)
+            if (int rc = h[i].ensure(std::max<uint64_t>(n, 1) * elem_bytes[i])) return rc;
+        if (n) {
+            for (int i = 0; i < count(keys); i++) {
+                CK(cudaMemcpyAsync(h[i].p, d[i].p, n * elem_bytes[i], cudaMemcpyDeviceToHost, s));
+                bytes += n * elem_bytes[i];
+            }
+            CK(cudaStreamSynchronize(s));
+        }
+        r.first_pos = h[FIRST_POS].as<uint64_t>(); r.frequency = h[FREQUENCY].as<uint16_t>();
+        r.out_deg = h[OUT_DEG].as<uint8_t>(); r.in_deg = h[IN_DEG].as<uint8_t>();
+        r.out_succ = h[OUT_SUCC].as<uint32_t>(); r.in_pred = h[IN_PRED].as<uint32_t>();
+        r.kmer_lo = keys ? h[KMER_LO].as<uint64_t>() : nullptr; r.kmer_hi = keys ? h[KMER_HI].as<uint64_t>() : nullptr;
+        return 0;
+    }
+};
+
+/* Events recorded on the context's stream, named after the point of the build they mark */
+enum Ev {
+    EV_BUILD,                                /* start of the build's device time (run_plan) */
+    EV_SCATTER, EV_SCATTER_END,              /* around k_scatter */
+    EV_INIT1, EV_PASS1, EV_PRUNE, EV_PRUNE_END,   /* before k_init_table1, k_pass1, k_prune; after k_prune */
+    EV_TABLE2, EV_PASS2, EV_PASS2_END,       /* before the survivor table, before k_pass2, after k_pass2 */
+    /* the finish, from its start to its end; a distributed finish records after each of its three steps and
+     * after the barrier behind it (the order is the order on the stream) */
+    EV_FINISH, EV_STEP0, EV_STEP0_MET, EV_STEP1, EV_STEP1_MET, EV_STEP2, EV_STEP2_MET, EV_FINISH_END,
+    EV_HASHMAP, EV_HASHMAP_END,              /* around the hash-map layout */
+    EV_COUNT
+};
+static_assert(EV_FINISH_END == EV_FINISH + 7, "the finish's events are consecutive");
 
 constexpr uint32_t STAGE_CHUNK = 32768; /* records per staging chunk (3.3 MB of text at L=50) */
 constexpr double MERGED_SLOTS_PER_NODE = 2.0;   /* slots of the merged survivor table per node (load 0.5) */
@@ -145,6 +215,10 @@ constexpr uint64_t SLICE_BYTES = 12ull << 20;   /* table-1 bytes one hash unit a
 enum { BUF_BASES = 0, BUF_VALID, BUF_QUAL, BUF_STRAND, BUF_TUPLES, BUF_GATHER, NBUF };
 static_assert(NBUF == VDJGRAPH_SHARD_NBUF, "header and library disagree");
 
+/* where a build stands: what has happened last.  FINISH_STEPn: step n of the finish has been queued or done
+ * (the three are consecutive, see finish_step_phase). */
+enum class Phase { STAGED, COUNTED, PLANNED, SCATTERED, PASSES_DONE, FINISH_PLANNED, FINISH_STEP0, FINISH_STEP1, FINISH_STEP2, FINISHED };
+
 struct Shard {
     int G = 1, rank = 0;
     uint64_t rec_base[MAX_DEV + 1] = {};
@@ -155,6 +229,7 @@ struct Shard {
     std::vector<double> est;                      /* [NU] distinct gated k-mers (HyperLogLog) */
     std::vector<int> owner, round_of;             /* [NU] device and round that process the unit */
     std::vector<UnitTab> utab;                    /* [NU] this device's table slices of the current round */
+    double load1 = 0;                             /* target load of table 1 (VDJGRAPH_LOAD1) */
     double slot_scale = 1.0;                      /* table-1 slots per estimated k-mer, relative to the default */
     bool ignore_hint = false;                     /* the caller's table_capacity turned out too small */
     void *peer[MAX_DEV][NBUF] = {};
@@ -169,9 +244,7 @@ struct Shard {
     float acc[6] = {};                            /* scatter, init1, pass1, prune, table2, pass2 ms summed over the rounds */
     bool merged() const { return G > 1 || S > 1; } /* the finish builds a table over survivor RECORDS */
     uint64_t bar_seq = 0;                         /* device barriers of this build so far (k_peer_barrier) */
-    /* 0 staged, 1 counted, 2 planned, 3 scattered, 4 passes done, 5 finish planned, 6 / 7 / 8 finish step 1 / 2 / 3
-     * queued or done, 9 finished */
-    int phase = 0;
+    Phase phase = Phase::STAGED;
 };
 
 struct vdjgraph_ctx {
@@ -184,30 +257,30 @@ struct vdjgraph_ctx {
     bool any_strand1 = false;
     bool staged = false, ran = false, staged_direct = false;
     cudaStream_t stream = nullptr;
-    cudaEvent_t ev[13] = {};
+    cudaEvent_t ev[EV_COUNT] = {};
     std::vector<StageWorker> workers;
 
     DevBuf d_bad, d_bases, d_good, d_valid, d_hiq, d_qual, d_strand;
     PinBuf h_bad;
     DevBuf d_t1, d_log, d_t2, d_hll, d_ctr, d_hist, d_cursor, d_tuples, d_utab;
     DevBuf d_keys[2], d_vals[2], d_cub;
-    DevBuf d_first_pos, d_freq, d_odeg, d_ideg, d_osucc, d_ipred, d_klo, d_khi;
+    NodeArrays nodes;
     DevBuf d_pre_klo, d_pre_khi, d_pre_freq, d_pre_n;
     PinBuf h_ctr, h_hll, h_hist, h_cursor, h_utab;
     float ms_count = 0;
     size_t count_smem = 0;
     int count_bps = 1;
     Part part;
-    PinBuf h_first_pos, h_freq, h_odeg, h_ideg, h_osucc, h_ipred, h_klo, h_khi;
     PinBuf h_pre_klo, h_pre_khi, h_pre_freq, h_pre_n;
 
     DevBuf d_tbase, d_rec, d_gather, d_t2m, d_gid, d_owner;
     DevBuf d_hm_hash, d_hm_probe, d_hm_prev, d_hm_owner, d_hm_slots, d_hm_flag;
     PinBuf h_hm_slots, h_hm_flag;
-    cudaEvent_t ev_hm[2] = {};
-    cudaEvent_t ev_fin[6] = {};                   /* after each step of a distributed finish and after the barrier behind it */
     PinBuf h_tbase;
     Shard sh;
+
+    /* the buffers that peers of a sharded build map, in BUF_* order */
+    std::array<DevBuf *, NBUF> peer_bufs() { return { &d_bases, &d_valid, &d_qual, &d_strand, &d_tuples, &d_gather }; }
 
     uint64_t cap1 = 0, cap2 = 0;
     uint32_t log_cap = 0;
@@ -269,8 +342,7 @@ int ensure_workers(vdjgraph_ctx *c, int n) {
     c->workers.resize(n);
     for (size_t i = old; i < c->workers.size(); i++) {
         CK(cudaStreamCreateWithFlags(&c->workers[i].stream, cudaStreamNonBlocking));
-        CK(cudaEventCreateWithFlags(&c->workers[i].ev[0], cudaEventDisableTiming));
-        CK(cudaEventCreateWithFlags(&c->workers[i].ev[1], cudaEventDisableTiming));
+        for (cudaEvent_t &e : c->workers[i].done) CK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
     }
     return 0;
 }
@@ -285,6 +357,22 @@ uint64_t chunk_records(const vdjgraph_ctx *c, uint32_t base) {
     return std::max<uint64_t>(tr, (base / tr) * tr);
 }
 int count_chunk(vdjgraph_ctx *c, cudaStream_t s, uint64_t rec_lo, uint64_t rec_hi, bool last);
+
+/* queues k_pack of text records [r_lo, r_hi) of R, whose text is at `text` on the device, and k_count of
+ * the packed records behind it on stream s */
+int pack_chunk(vdjgraph_ctx *c, cudaStream_t s, const unsigned char *text, uint64_t r_lo, uint64_t r_hi, uint64_t R, uint32_t fwd) {
+    const uint64_t n = r_hi - r_lo;
+    PackArgs pa;
+    pa.text = text; pa.r0 = r_lo << fwd; pa.n = n; pa.fwd_only = fwd;
+    pa.bases = c->d_bases.as<u64>(); pa.good = c->d_good.as<u64>(); pa.valid = c->d_valid.as<u64>();
+    pa.hiq = c->d_hiq.as<u64>();
+    pa.qual = c->d_qual.as<u8>(); pa.strand = c->d_strand.as<u8>();
+    pa.bad = c->d_bad.as<u64>();
+    const int grid = (int)std::min<uint64_t>((n + WARPS - 1) / WARPS, (uint64_t)c->sm_count * 8);
+    k_pack<<<grid, THREADS, 0, s>>>(pa, c->g);
+    CK(cudaGetLastError());
+    return count_chunk(c, s, r_lo << fwd, r_hi << fwd, r_hi == R);
+}
 
 struct StageShared {
     vdjgraph_ctx *c;
@@ -309,7 +397,7 @@ void stage_worker(StageShared *s, int wi) {
         if (ch >= n_chunks || s->status.load() != 0) break;
         const uint64_t r_lo = ch * CH, r_hi = std::min<uint64_t>(s->R, r_lo + CH);
         const uint64_t n = r_hi - r_lo;
-        if (w.busy[b]) { cudaEventSynchronize(w.ev[b]); w.busy[b] = false; }
+        if (w.busy[b]) { cudaEventSynchronize(w.done[b]); w.busy[b] = false; }
         char *pin = w.buf[b].as<char>();
         /* records [r_lo, r_hi) of primary ++ secondary */
         const uint64_t np_part = r_lo < s->np ? std::min<uint64_t>(r_hi, s->np) - r_lo : 0;
@@ -318,19 +406,8 @@ void stage_worker(StageShared *s, int wi) {
         /* stream order keeps the chunk's previous k_pack ahead of this copy */
         unsigned char *dst = w.dbuf[b].as<unsigned char>();
         cudaError_t e = cudaMemcpyAsync(dst, pin, n * rec_len, cudaMemcpyHostToDevice, w.stream);
-        if (e == cudaSuccess) {
-            PackArgs pa;
-            pa.text = dst; pa.r0 = r_lo << s->fwd; pa.n = n; pa.fwd_only = s->fwd;
-            pa.bases = c->d_bases.as<u64>(); pa.good = c->d_good.as<u64>(); pa.valid = c->d_valid.as<u64>();
-            pa.hiq = c->d_hiq.as<u64>();
-            pa.qual = c->d_qual.as<u8>(); pa.strand = c->d_strand.as<u8>();
-            pa.bad = c->d_bad.as<u64>();
-            const int grid = (int)std::min<uint64_t>((n + WARPS - 1) / WARPS, (uint64_t)c->sm_count * 8);
-            k_pack<<<grid, THREADS, 0, w.stream>>>(pa, g);
-            e = cudaGetLastError();
-            if (e == cudaSuccess && count_chunk(c, w.stream, r_lo << s->fwd, r_hi << s->fwd, r_hi == s->R)) e = cudaErrorUnknown;
-        }
-        if (e == cudaSuccess) e = cudaEventRecord(w.ev[b], w.stream);
+        if (e == cudaSuccess && pack_chunk(c, w.stream, dst, r_lo, r_hi, s->R, s->fwd)) e = cudaErrorUnknown;
+        if (e == cudaSuccess) e = cudaEventRecord(w.done[b], w.stream);
         if (e != cudaSuccess) { s->status = VDJGRAPH_ERR_CUDA; break; }
         w.busy[b] = true;
         b ^= 1;
@@ -374,18 +451,36 @@ int stage_direct(vdjgraph_ctx *c, const char *primary, uint64_t np, const char *
         if (np_part < n)
             CK(cudaMemcpyAsync(dst + np_part * rec_len, secondary + (r_lo + np_part - np) * rec_len, (n - np_part) * rec_len,
                                cudaMemcpyHostToDevice, w.stream));
-        PackArgs pa;
-        pa.text = dst; pa.r0 = r_lo << fwd; pa.n = n; pa.fwd_only = fwd;
-        pa.bases = c->d_bases.as<u64>(); pa.good = c->d_good.as<u64>(); pa.valid = c->d_valid.as<u64>();
-        pa.hiq = c->d_hiq.as<u64>();
-        pa.qual = c->d_qual.as<u8>(); pa.strand = c->d_strand.as<u8>();
-        pa.bad = c->d_bad.as<u64>();
-        const int grid = (int)std::min<uint64_t>((n + WARPS - 1) / WARPS, (uint64_t)c->sm_count * 8);
-        k_pack<<<grid, THREADS, 0, w.stream>>>(pa, g);
-        CK(cudaGetLastError());
-        if ((rc = count_chunk(c, w.stream, r_lo << fwd, r_hi << fwd, r_hi == R))) return rc;
+        if ((rc = pack_chunk(c, w.stream, dst, r_lo, r_hi, R, fwd))) return rc;
     }
     for (int i = 0; i < DIRECT_STREAMS; i++) CK(cudaStreamSynchronize(c->workers[i].stream));
+    return 0;
+}
+
+/* Staging from pageable caller buffers: up to host_threads workers (stage_worker) */
+int stage_pageable(vdjgraph_ctx *c, const char *primary, uint64_t np, const char *secondary, uint64_t R, uint32_t fwd) {
+    const size_t rec_len = (size_t)2 * c->g.L + 1;
+    const uint64_t CH = chunk_records(c, STAGE_CHUNK);
+    const uint64_t n_chunks = (R + CH - 1) / CH;
+    int nt = c->prm.host_threads > 0 ? c->prm.host_threads : (int)std::min(16u, std::thread::hardware_concurrency());
+    nt = std::max(1, std::min<int>(nt, 64));
+    nt = (int)std::min<uint64_t>((uint64_t)nt, n_chunks);
+    int rc;
+    if ((rc = ensure_workers(c, nt))) return rc;
+    for (int i = 0; i < nt; i++)
+        for (int b = 0; b < 2; b++)
+            if ((rc = c->workers[i].buf[b].ensure((size_t)CH * rec_len)) ||
+                (rc = c->workers[i].dbuf[b].ensure((size_t)CH * rec_len))) return rc;
+    StageShared sh;
+    sh.c = c; sh.primary = primary; sh.secondary = secondary; sh.np = np; sh.R = R; sh.fwd = fwd;
+    std::vector<std::thread> th;
+    for (int i = 1; i < nt; i++) th.emplace_back(stage_worker, &sh, i);
+    stage_worker(&sh, 0);
+    for (auto &t : th) t.join();
+    if (int st = sh.status.load()) {
+        cudaError_t e = cudaGetLastError();
+        return fail(st, "staging failed: %s", cudaGetErrorString(e));
+    }
     return 0;
 }
 
@@ -457,10 +552,8 @@ extern "C" int vdjgraph_create(const vdjgraph_params *params, vdjgraph_ctx **out
     memset(&c->res, 0, sizeof(c->res));
     memset(&c->ctr, 0, sizeof(c->ctr));
     e = cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking);
-    for (int i = 0; i < 13 && e == cudaSuccess; i++) e = cudaEventCreate(&c->ev[i]);
-    for (int i = 0; i < 2 && e == cudaSuccess; i++) e = cudaEventCreate(&c->ev_hm[i]);
-    for (int i = 0; i < 6 && e == cudaSuccess; i++) e = cudaEventCreate(&c->ev_fin[i]);
-    if (e != cudaSuccess) { delete c; return fail(VDJGRAPH_ERR_CUDA, "stream/event creation failed: %s", cudaGetErrorString(e)); }
+    for (cudaEvent_t &ev : c->ev) if (e == cudaSuccess) e = cudaEventCreate(&ev);
+    if (e != cudaSuccess) { vdjgraph_destroy(c); return fail(VDJGRAPH_ERR_CUDA, "stream/event creation failed: %s", cudaGetErrorString(e)); }
     *out = c;
     return 0;
 }
@@ -470,25 +563,12 @@ extern "C" void vdjgraph_destroy(vdjgraph_ctx *c) {
     cudaSetDevice(c->device);
     cudaDeviceSynchronize();
     for (auto &w : c->workers) {
-        w.buf[0].release(); w.buf[1].release();
-        w.dbuf[0].release(); w.dbuf[1].release();
-        if (w.ev[0]) cudaEventDestroy(w.ev[0]);
-        if (w.ev[1]) cudaEventDestroy(w.ev[1]);
+        for (cudaEvent_t ev : w.done) if (ev) cudaEventDestroy(ev);
         if (w.stream) cudaStreamDestroy(w.stream);
     }
-    DevBuf *db[] = { &c->d_hm_hash, &c->d_hm_probe, &c->d_hm_prev, &c->d_hm_owner, &c->d_hm_slots, &c->d_hm_flag, &c->d_hiq, &c->d_tbase, &c->d_rec, &c->d_gather, &c->d_t2m, &c->d_gid, &c->d_owner, &c->d_bad, &c->d_bases, &c->d_good, &c->d_valid, &c->d_qual, &c->d_strand, &c->d_t1, &c->d_log, &c->d_t2,
-                     &c->d_hll, &c->d_ctr, &c->d_hist, &c->d_cursor, &c->d_tuples, &c->d_utab, &c->d_keys[0], &c->d_keys[1], &c->d_vals[0], &c->d_vals[1], &c->d_cub,
-                     &c->d_first_pos, &c->d_freq, &c->d_odeg, &c->d_ideg, &c->d_osucc, &c->d_ipred, &c->d_klo,
-                     &c->d_khi, &c->d_pre_klo, &c->d_pre_khi, &c->d_pre_freq, &c->d_pre_n };
-    for (DevBuf *b : db) b->release();
-    PinBuf *pb[] = { &c->h_hm_slots, &c->h_hm_flag, &c->h_utab, &c->h_tbase, &c->h_bad, &c->h_ctr, &c->h_hll, &c->h_hist, &c->h_cursor, &c->h_first_pos, &c->h_freq, &c->h_odeg, &c->h_ideg, &c->h_osucc,
-                     &c->h_ipred, &c->h_klo, &c->h_khi, &c->h_pre_klo, &c->h_pre_khi, &c->h_pre_freq, &c->h_pre_n };
-    for (PinBuf *b : pb) b->release();
-    for (int i = 0; i < 13; i++) if (c->ev[i]) cudaEventDestroy(c->ev[i]);
-    for (int i = 0; i < 2; i++) if (c->ev_hm[i]) cudaEventDestroy(c->ev_hm[i]);
-    for (int i = 0; i < 6; i++) if (c->ev_fin[i]) cudaEventDestroy(c->ev_fin[i]);
+    for (cudaEvent_t ev : c->ev) if (ev) cudaEventDestroy(ev);
     if (c->stream) cudaStreamDestroy(c->stream);
-    delete c;
+    delete c;   /* the buffers free themselves */
 }
 
 extern "C" int vdjgraph_set_params(vdjgraph_ctx *c, const vdjgraph_params *params) {
@@ -545,30 +625,7 @@ static int stage_impl(vdjgraph_ctx *c, const char *primary, size_t np, const cha
         CK(cudaMemcpyAsync(c->d_bad.p, hb, 3 * sizeof(uint64_t), cudaMemcpyHostToDevice, c->stream));
         CK(cudaStreamSynchronize(c->stream));   /* padding memsets, flags and zeroed counters are in place before the workers start */
         const bool direct = is_page_locked(primary, np * rec_len) && is_page_locked(secondary, ns * rec_len);
-        if (direct) {
-            if ((rc = stage_direct(c, primary, np, secondary, Rt, fwd))) return rc;
-        } else {
-        const uint64_t CH = chunk_records(c, STAGE_CHUNK);
-        const uint64_t n_chunks = (Rt + CH - 1) / CH;
-        int nt = c->prm.host_threads > 0 ? c->prm.host_threads : (int)std::min(16u, std::thread::hardware_concurrency());
-        nt = std::max(1, std::min<int>(nt, 64));
-        nt = (int)std::min<uint64_t>((uint64_t)nt, n_chunks);
-        if ((rc = ensure_workers(c, nt))) return rc;
-        for (int i = 0; i < nt; i++)
-            for (int b = 0; b < 2; b++)
-                if ((rc = c->workers[i].buf[b].ensure((size_t)CH * rec_len)) ||
-                    (rc = c->workers[i].dbuf[b].ensure((size_t)CH * rec_len))) return rc;
-        StageShared sh;
-        sh.c = c; sh.primary = primary; sh.secondary = secondary; sh.np = np; sh.R = Rt; sh.fwd = fwd;
-        std::vector<std::thread> th;
-        for (int i = 1; i < nt; i++) th.emplace_back(stage_worker, &sh, i);
-        stage_worker(&sh, 0);
-        for (auto &t : th) t.join();
-        if (int st = sh.status.load()) {
-            cudaError_t e = cudaGetLastError();
-            return fail(st, "staging failed: %s", cudaGetErrorString(e));
-        }
-        }
+        if ((rc = direct ? stage_direct(c, primary, np, secondary, Rt, fwd) : stage_pageable(c, primary, np, secondary, Rt, fwd))) return rc;
         c->staged_direct = direct;
         CK(cudaMemcpyAsync(hb, c->d_bad.p, 3 * sizeof(uint64_t), cudaMemcpyDeviceToHost, c->stream));
         CK(cudaStreamSynchronize(c->stream));
@@ -612,11 +669,43 @@ extern "C" int vdjgraph_stage_forward(vdjgraph_ctx *c, const char *primary_reads
 namespace {
 
 
-int phase_check(vdjgraph_ctx *c, int want, const char *what) {
+int phase_check(vdjgraph_ctx *c, Phase want, const char *what) {
     if (!c) return fail(VDJGRAPH_ERR_PARAM, "ctx is NULL");
     if (!c->staged) return fail(VDJGRAPH_ERR_STATE, "%s before vdjgraph_stage", what);
-    if (c->sh.phase != want) return fail(VDJGRAPH_ERR_STATE, "%s called in phase %d (expected %d)", what, c->sh.phase, want);
+    if (c->sh.phase != want) return fail(VDJGRAPH_ERR_STATE, "%s called in phase %d (expected %d)", what, (int)c->sh.phase, (int)want);
     return 0;
+}
+
+/* the phase once finish step `step` (0, 1, 2) has been queued */
+Phase finish_step_phase(int step) { return Phase((int)Phase::FINISH_STEP0 + step); }
+
+/* the device counters to the host (c->h_ctr), the stream synchronised */
+int read_counters(vdjgraph_ctx *c) {
+    CK(cudaMemcpyAsync(c->h_ctr.p, c->d_ctr.p, sizeof(Counters), cudaMemcpyDeviceToHost, c->stream));
+    CK(cudaStreamSynchronize(c->stream));
+    return 0;
+}
+
+/* adds this round's kernel times (scatter, init1, pass1, prune, table2, pass2) into sh.acc; every event
+ * of the round has completed */
+void add_kernel_times(vdjgraph_ctx *c) {
+    static const Ev span[6][2] = { { EV_SCATTER, EV_SCATTER_END }, { EV_INIT1, EV_PASS1 }, { EV_PASS1, EV_PRUNE },
+                                   { EV_PRUNE, EV_PRUNE_END }, { EV_TABLE2, EV_PASS2 }, { EV_PASS2, EV_PASS2_END } };
+    for (int i = 0; i < 6; i++) {
+        float ms = 0;
+        cudaEventElapsedTime(&ms, c->ev[span[i][0]], c->ev[span[i][1]]);
+        c->sh.acc[i] += ms;
+    }
+}
+
+/* this device's times once the finish has completed: per kernel, summed over the rounds (k_count ran with
+ * the staging: ms_estimate), the hash-map layout and the finish */
+void take_times(vdjgraph_ctx *c) {
+    vdjgraph_result &res = c->res;
+    const float *acc = c->sh.acc;
+    res.ms_scatter = acc[0]; res.ms_init1 = acc[1]; res.ms_pass1 = acc[2]; res.ms_prune = acc[3]; res.ms_table2 = acc[4]; res.ms_pass2 = acc[5];
+    if (res.hm_buckets) cudaEventElapsedTime(&res.ms_hashmap, c->ev[EV_HASHMAP], c->ev[EV_HASHMAP_END]);
+    cudaEventElapsedTime(&res.ms_export, c->ev[EV_FINISH], c->ev[EV_FINISH_END]);
 }
 
 constexpr size_t HIST_WORDS = 3 * NBUCKET;          /* runs | gated windows | N-free windows, per bucket */
@@ -683,10 +772,10 @@ void reset_run_stats(vdjgraph_ctx *c) {
 }
 
 /* table-1 slots of hash unit u (all of it, whichever device / round holds it) */
-uint64_t unit_slots1(const Shard &sh, const vdjgraph_params &prm, int u, double load1) {
+uint64_t unit_slots1(const Shard &sh, const vdjgraph_params &prm, int u) {
     /* 1.15: the per-unit HyperLogLog has a relative error of ~9 % / sqrt(buckets per unit); a slice that
      * comes out too small only runs at a higher load (probing continues into the next slice) */
-    double slots = sh.est[u] * 1.15 / load1 * sh.slot_scale;
+    double slots = sh.est[u] * 1.15 / sh.load1 * sh.slot_scale;
     if (prm.table_capacity && !sh.ignore_hint) slots = (double)prm.table_capacity * (sh.est[u] + 1.0) / (sh.est_distinct + sh.NU) * sh.slot_scale;
     return (uint64_t)slots + 64;
 }
@@ -700,19 +789,17 @@ int run_plan(vdjgraph_ctx *c, const uint64_t *hist_all, const uint8_t *hll) {
     const Geom &g = c->g;
     const int G = sh.G;
     reset_run_stats(c);
-    CK(cudaEventRecord(c->ev[0], c->stream));   /* start of the device time of this build */
+    CK(cudaEventRecord(c->ev[EV_BUILD], c->stream));
     /* per-bucket estimates of the distinct gated k-mers */
     double est_b[NBUCKET];
-    uint64_t gated_total = 0;
     sh.est_distinct = 0;
     for (int b = 0; b < NBUCKET; b++) {
         uint64_t gb = 0;
         for (int d = 0; d < G; d++) gb += hist_all[((size_t)d * 3 + 1) * NBUCKET + b];
         est_b[b] = gb ? std::min<double>(hll_estimate(hll + (size_t)b * BHLL), (double)gb) : 0.0;
         sh.est_distinct += est_b[b];
-        gated_total += gb;
     }
-    const double load1 = std::min(0.9, std::max(0.05, env_double("VDJGRAPH_LOAD1", 0.5)));
+    const double load1 = sh.load1 = std::min(0.9, std::max(0.05, env_double("VDJGRAPH_LOAD1", 0.5)));
     const uint64_t cap1_all = c->prm.table_capacity ? c->prm.table_capacity : (uint64_t)(sh.est_distinct * 1.15 / load1) + 1024;
 
     Part pt;
@@ -796,7 +883,7 @@ int run_plan(vdjgraph_ctx *c, const uint64_t *hist_all, const uint8_t *hll) {
             sh.round_of[u] = best;
             load_rnd[(size_t)d * S + best] += tot_runs[u] + 1;
             gated_rnd[(size_t)d * S + best] += tot_gated[u];
-            est_rnd[(size_t)d * S + best] += (double)unit_slots1(sh, c->prm, u, load1);
+            est_rnd[(size_t)d * S + best] += (double)unit_slots1(sh, c->prm, u);
         }
     };
     const bool free_tables = env_double("VDJGRAPH_FREE_TABLES_MB", -1.0) >= 0;
@@ -859,19 +946,16 @@ int run_plan(vdjgraph_ctx *c, const uint64_t *hist_all, const uint8_t *hll) {
     c->res.tuple_bytes = (uint32_t)(pt.wide ? 24 : 16);
     c->res.rounds = (uint32_t)sh.S;
     c->res.n_gated = sh.n_gated_src;
-    uint64_t all_runs = 0, all_valid = 0;
-    for (int u = 0; u < sh.NU; u++) { all_runs += tot_runs[u]; all_valid += tot_valid[u]; }
     c->res.n_runs = 0;
     for (int u = 0; u < sh.NU; u++) c->res.n_runs += sh.runs[(size_t)sh.rank * sh.NU + u];
     c->res.run_bytes = (uint32_t)(RUN_WORDS * 8);
-    (void)all_runs; (void)all_valid; (void)gated_total;
     sh.peers_set = false;
-    sh.phase = 2;
+    sh.phase = Phase::PLANNED;
     return 0;
 }
 
 void own_buffers(vdjgraph_ctx *c, void **ptrs, size_t *bytes) {
-    DevBuf *b[NBUF] = { &c->d_bases, &c->d_valid, &c->d_qual, &c->d_strand, &c->d_tuples, &c->d_gather };
+    const auto b = c->peer_bufs();
     for (int i = 0; i < NBUF; i++) { ptrs[i] = b[i]->p; if (bytes) bytes[i] = b[i]->cap; }
 }
 
@@ -920,7 +1004,7 @@ int run_scatter(vdjgraph_ctx *c) {
     CK(cudaMemcpyAsync(c->d_cursor.p, cur, 2 * NBUCKET * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
     CK(cudaMemcpyAsync(c->d_tbase.p, tb, NBUCKET * sizeof(void *), cudaMemcpyHostToDevice, s));
     CK(cudaMemsetAsync(c->d_ctr.p, 0, sizeof(Counters), s));
-    CK(cudaEventRecord(c->ev[10], s));
+    CK(cudaEventRecord(c->ev[EV_SCATTER], s));
     if (g.R) {
         ScatterArgs as;
         as.bases = c->d_bases.as<u64>(); as.good = c->d_good.as<u64>(); as.valid = c->d_valid.as<u64>();
@@ -935,9 +1019,9 @@ int run_scatter(vdjgraph_ctx *c) {
         c->res.kernel_launches++;
         CK(cudaGetLastError());
     }
-    CK(cudaEventRecord(c->ev[11], s));
+    CK(cudaEventRecord(c->ev[EV_SCATTER_END], s));
     if (G > 1) CK(cudaStreamSynchronize(s));   /* the peers' runs are complete once every device got here */
-    sh.phase = 3;
+    sh.phase = Phase::SCATTERED;
     return 0;
 }
 
@@ -970,7 +1054,6 @@ int run_passes(vdjgraph_ctx *c) {
     const uint64_t n_runs = pt.n_runs, n_gated = sh.n_gated_own;
     const Reads rd = make_reads(c);
     const int grid_flat = c->sm_count * 8;
-    const double load1 = std::min(0.9, std::max(0.05, env_double("VDJGRAPH_LOAD1", 0.5)));
 
     /* pruning constants: T = min(mq, 214) after the <=254 clamp (:1514-1516, :356-360);
      * NB = ceil(T/20) = largest count whose quality sums can still fail */
@@ -998,7 +1081,7 @@ int run_passes(vdjgraph_ctx *c) {
         cap1 = 0;
         for (int u = 0; u < sh.NU; u++) {
             if (sh.owner[u] != sh.rank || sh.round_of[u] != sh.rnd) continue;
-            const uint64_t len = unit_slots1(sh, c->prm, u, load1);
+            const uint64_t len = unit_slots1(sh, c->prm, u);
             if (cap1 + len > 0xFFFFFFF0ull) return fail(VDJGRAPH_ERR_TOO_MANY_NODES, "pass-1 table would need more than 2^32 slots");
             sh.utab[u].off1 = (u32)cap1; sh.utab[u].len1 = (u32)len;
             cap1 += len;
@@ -1021,9 +1104,9 @@ int run_passes(vdjgraph_ctx *c) {
         CK(cudaMemcpyAsync(c->d_utab.p, ut, sh.NU * sizeof(UnitTab), cudaMemcpyHostToDevice, s));
 
         if (attempt) CK(cudaMemsetAsync(d_ctr, 0, sizeof(Counters), s));   /* first attempt: zeroed before the scatter */
-        CK(cudaEventRecord(c->ev[9], s));
+        CK(cudaEventRecord(c->ev[EV_INIT1], s));
         k_init_table1<<<grid_flat, THREADS, 0, s>>>(c->d_t1.as<Slot1>(), cap1);
-        CK(cudaEventRecord(c->ev[2], s));
+        CK(cudaEventRecord(c->ev[EV_PASS1], s));
         Pass1Args a1;
         a1.runs = c->d_tuples.as<u64>();
         a1.rd = rd;
@@ -1032,16 +1115,15 @@ int run_passes(vdjgraph_ctx *c) {
         a1.ctr = d_ctr;
         if (pt.wide) k_pass1<true><<<grid_p1, THREADS, smem_q1, s>>>(a1, g, pt);
         else k_pass1<false><<<grid_p1, THREADS, smem_q1, s>>>(a1, g, pt);
-        CK(cudaEventRecord(c->ev[3], s));
+        CK(cudaEventRecord(c->ev[EV_PRUNE], s));
         PruneArgs ap;
         ap.table = c->d_t1.as<Slot1>(); ap.cap = cap1; ap.log = c->d_log.as<u64>(); ap.nb_ranks = (uint32_t)NB;
         ap.rd = rd; ap.mf = c->prm.min_node_freq; ap.T = T; ap.ctr = d_ctr;
         k_prune<<<grid_flat, THREADS, 0, s>>>(ap, g);
-        CK(cudaEventRecord(c->ev[4], s));
+        CK(cudaEventRecord(c->ev[EV_PRUNE_END], s));
         res.kernel_launches += 3;
         CK(cudaGetLastError());
-        CK(cudaMemcpyAsync(h_ctr, d_ctr, sizeof(Counters), cudaMemcpyDeviceToHost, s));
-        CK(cudaStreamSynchronize(s));
+        if ((rc = read_counters(c))) return rc;
         if (h_ctr->overflow == 4) return fail(VDJGRAPH_ERR_INTERNAL, "run region overrun in k_scatter");
         if (h_ctr->overflow == 2) { log_scale *= 2.0; continue; }   /* the occurrence log ran out of blocks */
         if (h_ctr->overflow) {   /* table full or a probe chain past MAX_PROBE: a too small hint is dropped, else more room */
@@ -1081,16 +1163,16 @@ int run_passes(vdjgraph_ctx *c) {
     c->cap2 = cap2;
     memcpy(ut, sh.utab.data(), sh.NU * sizeof(UnitTab));
     CK(cudaMemcpyAsync(c->d_utab.p, ut, sh.NU * sizeof(UnitTab), cudaMemcpyHostToDevice, s));
-    CK(cudaEventRecord(c->ev[5], s));
+    CK(cudaEventRecord(c->ev[EV_TABLE2], s));
     k_init_table2<<<grid_flat, THREADS, 0, s>>>(c->d_t2.as<Slot2>(), cap2);
     k_build_table2<<<grid_flat, THREADS, 0, s>>>(c->d_t1.as<Slot1>(), cap1, c->d_t2.as<Slot2>(), cap2, g, pt, d_ctr);
-    CK(cudaEventRecord(c->ev[6], s));
+    CK(cudaEventRecord(c->ev[EV_PASS2], s));
     Pass2Args a2;
     a2.runs = c->d_tuples.as<u64>();
     a2.table = c->d_t2.as<Slot2>(); a2.cap = cap2; a2.ctr = d_ctr;
     if (pt.wide) k_pass2<true><<<grid_p2, THREADS, smem_q, s>>>(a2, g, pt);
     else k_pass2<false><<<grid_p2, THREADS, smem_q, s>>>(a2, g, pt);
-    CK(cudaEventRecord(c->ev[7], s));
+    CK(cudaEventRecord(c->ev[EV_PASS2_END], s));
     res.kernel_launches += 3;
     CK(cudaGetLastError());
     res.table1_slots = cap1; res.table2_slots = cap2;
@@ -1104,26 +1186,19 @@ int run_passes(vdjgraph_ctx *c) {
         CK(cudaMemsetAsync(&d_ctr->n_nodes, 0, sizeof(u64), s));
         k_compact_table2<<<grid_flat, THREADS, 0, s>>>(c->d_t2.as<Slot2>(), cap2, c->d_rec.as<Slot2>() + done, &d_ctr->n_nodes);
         res.kernel_launches++;
-        CK(cudaMemcpyAsync(h_ctr, d_ctr, sizeof(Counters), cudaMemcpyDeviceToHost, s));
-        CK(cudaStreamSynchronize(s));
+        if ((rc = read_counters(c))) return rc;
         if (h_ctr->overflow) return fail(VDJGRAPH_ERR_INTERNAL, "survivor table overflow (code %u)", h_ctr->overflow);
         if (h_ctr->n_nodes != n_surv) return fail(VDJGRAPH_ERR_INTERNAL, "compacted %llu survivors, expected %llu", (unsigned long long)h_ctr->n_nodes, (unsigned long long)n_surv);
         res.n_hits += h_ctr->n_hits;
         res.n_slow2 += h_ctr->n_slow2;
         res.n_hits_ungated += h_ctr->n_hits_ungated;
         sh.surv_done = done + n_surv;
-        /* this round's kernel times (the stream is idle: every event has completed) */
-        const int pairs[6][2] = { { 10, 11 }, { 9, 2 }, { 2, 3 }, { 3, 4 }, { 5, 6 }, { 6, 7 } };
-        for (int i = 0; i < 6; i++) {
-            float ms = 0;
-            cudaEventElapsedTime(&ms, c->ev[pairs[i][0]], c->ev[pairs[i][1]]);
-            sh.acc[i] += ms;
-        }
+        add_kernel_times(c);
     } else {
         sh.surv_done = n_surv;
     }
     sh.surv_all[sh.rank] = sh.surv_done;
-    sh.phase = 4;
+    sh.phase = Phase::PASSES_DONE;
     return 0;
 }
 
@@ -1135,7 +1210,7 @@ int run_hashmap_layout(vdjgraph_ctx *c, uint64_t n) {
     cudaStream_t s = c->stream;
     int rc;
     vdjgraph_result &res = c->res;
-    CK(cudaEventRecord(c->ev_hm[0], s));
+    CK(cudaEventRecord(c->ev[EV_HASHMAP], s));
     uint64_t final_buckets = 32;
     while (n > final_buckets / 2) final_buckets *= 2;
     if (final_buckets > (1ull << 32)) return fail(VDJGRAPH_ERR_TOO_MANY_NODES, "hash-map layout for %llu nodes", (unsigned long long)n);
@@ -1145,7 +1220,8 @@ int run_hashmap_layout(vdjgraph_ctx *c, uint64_t n) {
         (rc = c->d_hm_flag.ensure(16)) || (rc = c->h_hm_flag.ensure(16)))
         return rc;
     const int gb = (int)((na + THREADS - 1) / THREADS);
-    if (n) k_hm_hash<<<gb, THREADS, 0, s>>>(c->d_klo.as<u64>(), c->d_khi.as<u64>(), n, c->g.k, c->d_hm_hash.as<u64>());
+    if (n) k_hm_hash<<<gb, THREADS, 0, s>>>(c->nodes.d[NodeArrays::KMER_LO].as<u64>(), c->nodes.d[NodeArrays::KMER_HI].as<u64>(), n, c->g.k,
+                                            c->d_hm_hash.as<u64>());
     HmStage st;
     st.hash = c->d_hm_hash.as<u64>(); st.owner = c->d_hm_owner.as<u64>(); st.probe = c->d_hm_probe.as<u32>();
     st.prev_bucket = c->d_hm_prev.as<u32>(); st.changed = c->d_hm_flag.as<u32>();
@@ -1174,7 +1250,7 @@ int run_hashmap_layout(vdjgraph_ctx *c, uint64_t n) {
     }
     k_hm_slots<<<(int)((T + THREADS - 1) / THREADS), THREADS, 0, s>>>(st.owner, T, c->d_hm_slots.as<u32>());
     CK(cudaGetLastError());
-    CK(cudaEventRecord(c->ev_hm[1], s));
+    CK(cudaEventRecord(c->ev[EV_HASHMAP_END], s));
     res.hm_buckets = T;
     return 0;
 }
@@ -1194,7 +1270,7 @@ int run_finish(vdjgraph_ctx *c) {
     uint64_t n_surv = sh.surv_all[sh.rank];
     uint64_t cap2 = c->cap2;
     Slot2 *table = c->d_t2.as<Slot2>();
-    CK(cudaEventRecord(c->ev[12], s));
+    CK(cudaEventRecord(c->ev[EV_FINISH], s));
     if (sh.merged()) {
         /* several rounds on one device: the survivor records of all rounds */
         const Slot2 *records = c->d_rec.as<Slot2>();
@@ -1219,15 +1295,11 @@ int run_finish(vdjgraph_ctx *c) {
         res.kernel_launches += 2;
     }
     const size_t na = std::max<uint64_t>(n_surv, 1);
+    const bool keys = want_keys(c->prm.flags);
     if ((rc = c->d_keys[0].ensure(na * 8)) || (rc = c->d_keys[1].ensure(na * 8)) ||
         (rc = c->d_vals[0].ensure(na * 4)) || (rc = c->d_vals[1].ensure(na * 4)) ||
-        (rc = c->d_first_pos.ensure(na * 8)) || (rc = c->d_freq.ensure(na * 2)) ||
-        (rc = c->d_odeg.ensure(na)) || (rc = c->d_ideg.ensure(na)) ||
-        (rc = c->d_osucc.ensure(na * 16)) || (rc = c->d_ipred.ensure(na * 16)))
+        (rc = c->nodes.ensure(n_surv, keys)))
         return rc;
-    const bool want_layout = c->prm.flags & VDJGRAPH_FLAG_HASHMAP_LAYOUT;
-    const bool want_keys = (c->prm.flags & VDJGRAPH_FLAG_EXPORT_KEYS) || want_layout;   /* the layout hashes the nodes' k-mers */
-    if (want_keys && ((rc = c->d_klo.ensure(na * 8)) || (rc = c->d_khi.ensure(na * 8)))) return rc;
     const int end_bit = bits_for(sh.total_records * (uint64_t)g.w);
     size_t cub_bytes = 0;
     CK(cub::DeviceRadixSort::SortPairs(nullptr, cub_bytes, c->d_keys[0].as<u64>(), c->d_keys[1].as<u64>(),
@@ -1239,50 +1311,33 @@ int run_finish(vdjgraph_ctx *c) {
                                            c->d_vals[0].as<u32>(), c->d_vals[1].as<u32>(), (int64_t)n_surv, 0, end_bit, s));
         const int gb = (int)((n_surv + THREADS - 1) / THREADS);
         k_assign_rank<<<gb, THREADS, 0, s>>>(table, c->d_vals[1].as<u32>(), n_surv);
-        ExportArgs ae;
-        ae.table = table; ae.cap = cap2; ae.keys = c->d_keys[1].as<u64>(); ae.vals = c->d_vals[1].as<u32>();
-        ae.n = n_surv; ae.first_pos = c->d_first_pos.as<u64>(); ae.frequency = c->d_freq.as<u16>();
-        ae.out_deg = c->d_odeg.as<u8>(); ae.in_deg = c->d_ideg.as<u8>();
-        ae.out_succ = c->d_osucc.as<u32>(); ae.in_pred = c->d_ipred.as<u32>();
-        ae.kmer_lo = want_keys ? c->d_klo.as<u64>() : nullptr; ae.kmer_hi = want_keys ? c->d_khi.as<u64>() : nullptr;
+        ExportArgs ae = c->nodes.export_args(keys);
+        ae.table = table; ae.cap = cap2; ae.keys = c->d_keys[1].as<u64>(); ae.vals = c->d_vals[1].as<u32>(); ae.n = n_surv;
         k_export<<<gb, THREADS, 0, s>>>(ae, g, pt);
         res.kernel_launches += 3;
     }
     res.hm_buckets = 0; res.ms_hashmap = 0;
-    if (want_layout && (rc = run_hashmap_layout(c, n_surv))) return rc;
-    CK(cudaEventRecord(c->ev[8], s));
+    if ((c->prm.flags & VDJGRAPH_FLAG_HASHMAP_LAYOUT) && (rc = run_hashmap_layout(c, n_surv))) return rc;
+    CK(cudaEventRecord(c->ev[EV_FINISH_END], s));
     CK(cudaGetLastError());
-    CK(cudaMemcpyAsync(h_ctr, d_ctr, sizeof(Counters), cudaMemcpyDeviceToHost, s));
-    CK(cudaStreamSynchronize(s));
+    if ((rc = read_counters(c))) return rc;
     if (h_ctr->overflow) return fail(VDJGRAPH_ERR_INTERNAL, "survivor table overflow (code %u)", h_ctr->overflow);
     if (h_ctr->internal) return fail(VDJGRAPH_ERR_INTERNAL, "export invariant violated (code %u)", h_ctr->internal);
     if (n_surv && h_ctr->n_nodes != n_surv)
         return fail(VDJGRAPH_ERR_INTERNAL, "collected %llu nodes, expected %llu", (unsigned long long)h_ctr->n_nodes, (unsigned long long)n_surv);
     c->ctr = *h_ctr;
     res.n_nodes = n_surv;
-    if (res.hm_buckets) cudaEventElapsedTime(&res.ms_hashmap, c->ev_hm[0], c->ev_hm[1]);
     if (!sh.merged()) {
         res.n_hits = h_ctr->n_hits;
         res.n_slow2 = h_ctr->n_slow2;
         res.n_hits_ungated = h_ctr->n_hits_ungated;
+        add_kernel_times(c);   /* the only round (a merged build adds each round's in run_passes) */
     } else {
         res.n_pre = n_surv;
     }
-    /* per-kernel times of this device's share (k_count ran with the staging: ms_estimate) */
-    if (sh.merged()) {
-        res.ms_scatter = sh.acc[0]; res.ms_init1 = sh.acc[1]; res.ms_pass1 = sh.acc[2];
-        res.ms_prune = sh.acc[3]; res.ms_table2 = sh.acc[4]; res.ms_pass2 = sh.acc[5];
-    } else {
-        cudaEventElapsedTime(&res.ms_scatter, c->ev[10], c->ev[11]);
-        cudaEventElapsedTime(&res.ms_init1, c->ev[9], c->ev[2]);
-        cudaEventElapsedTime(&res.ms_pass1, c->ev[2], c->ev[3]);
-        cudaEventElapsedTime(&res.ms_prune, c->ev[3], c->ev[4]);
-        cudaEventElapsedTime(&res.ms_table2, c->ev[5], c->ev[6]);
-        cudaEventElapsedTime(&res.ms_pass2, c->ev[6], c->ev[7]);
-    }
-    cudaEventElapsedTime(&res.ms_export, c->ev[12], c->ev[8]);
-    cudaEventElapsedTime(&res.ms_device, c->ev[0], c->ev[8]);
-    sh.phase = 9;
+    take_times(c);
+    cudaEventElapsedTime(&res.ms_device, c->ev[EV_BUILD], c->ev[EV_FINISH_END]);
+    sh.phase = Phase::FINISHED;
     c->ran = true;
     return 0;
 }
@@ -1300,14 +1355,13 @@ FinishLayout finish_layout(const uint64_t *surv, int G, int rank, uint32_t flags
     f.n_total = 0;
     for (int d = 0; d < G; d++) f.n_total += surv[d];
     const uint64_t na = std::max<uint64_t>(f.n_total, 1);
-    const bool want_keys = flags & (VDJGRAPH_FLAG_EXPORT_KEYS | VDJGRAPH_FLAG_HASHMAP_LAYOUT);
     f.keys_off = FLAGS_BYTES;
     f.table_off = (f.keys_off + na * 8 + 255) & ~(size_t)255;
     f.cap = std::max<uint64_t>(1024, (uint64_t)((double)surv[rank] * MERGED_SLOTS_PER_NODE) + 64);
     f.rows_off = f.table_off + f.cap * sizeof(Slot2);
     f.over_off = f.rows_off + (rank == 0 ? na * ROW_WORDS * 8 : 0);
     f.kmers_off = f.over_off + (rank == 0 ? na * 16 : 0);
-    f.bytes = f.kmers_off + (rank == 0 && want_keys ? na * 16 : 0);
+    f.bytes = f.kmers_off + (rank == 0 && want_keys(flags) ? na * 16 : 0);
     return f;
 }
 RowSink row_sink(char *arena0, const FinishLayout &f0, uint32_t flags) {
@@ -1315,7 +1369,7 @@ RowSink row_sink(char *arena0, const FinishLayout &f0, uint32_t flags) {
     r.rows = reinterpret_cast<u64 *>(arena0 + f0.rows_off);
     r.over = reinterpret_cast<ulonglong2 *>(arena0 + f0.over_off);
     r.n_over = reinterpret_cast<u32 *>(arena0 + OVER_COUNT_OFF);
-    r.kmers = (flags & (VDJGRAPH_FLAG_EXPORT_KEYS | VDJGRAPH_FLAG_HASHMAP_LAYOUT)) ? reinterpret_cast<ulonglong2 *>(arena0 + f0.kmers_off) : nullptr;
+    r.kmers = want_keys(flags) ? reinterpret_cast<ulonglong2 *>(arena0 + f0.kmers_off) : nullptr;
     return r;
 }
 
@@ -1340,15 +1394,7 @@ int finish_plan(vdjgraph_ctx *c) {
     std::vector<u8> owner(NBUCKET, 0);
     for (int u = 0; u < sh.NU; u++) owner[u] = (u8)sh.owner[u];
     CK(cudaMemcpy(c->d_owner.p, owner.data(), NBUCKET, cudaMemcpyHostToDevice));
-    if (sh.rank == 0) {
-        const size_t na = std::max<uint64_t>(f.n_total, 1);
-        if ((rc = c->d_first_pos.ensure(na * 8)) || (rc = c->d_freq.ensure(na * 2)) || (rc = c->d_odeg.ensure(na)) ||
-            (rc = c->d_ideg.ensure(na)) || (rc = c->d_osucc.ensure(na * 16)) || (rc = c->d_ipred.ensure(na * 16)))
-            return rc;
-        if ((c->prm.flags & (VDJGRAPH_FLAG_EXPORT_KEYS | VDJGRAPH_FLAG_HASHMAP_LAYOUT)) &&
-            ((rc = c->d_klo.ensure(na * 8)) || (rc = c->d_khi.ensure(na * 8))))
-            return rc;
-    }
+    if (sh.rank == 0 && (rc = c->nodes.ensure(f.n_total, want_keys(c->prm.flags)))) return rc;
     return 0;
 }
 
@@ -1370,7 +1416,7 @@ int finish_step(vdjgraph_ctx *c, int step, bool device_barrier) {
     for (int d = 0; d < sh.G; d++)
         if (!sh.peer[d][BUF_GATHER]) return fail(VDJGRAPH_ERR_STATE, "device %d's exchange buffer is not set", d);
     if (step == 0) {
-        CK(cudaEventRecord(c->ev[12], s));
+        CK(cudaEventRecord(c->ev[EV_FINISH], s));
         Part pt = c->part;
         pt.flat = 1; pt.flat_len = (u32)f.cap;
         CK(cudaMemsetAsync(&d_ctr->n_nodes, 0, sizeof(u64), s));
@@ -1417,7 +1463,7 @@ int finish_step(vdjgraph_ctx *c, int step, bool device_barrier) {
         }
     }
     CK(cudaGetLastError());
-    CK(cudaEventRecord(c->ev_fin[2 * step], s));
+    CK(cudaEventRecord(c->ev[EV_STEP0 + 2 * step], s));
     if (device_barrier) {
         PeerFlags pf;
         for (int d = 0; d < MAX_DEV; d++) pf.flags[d] = reinterpret_cast<u64 *>(sh.peer[d < sh.G ? d : sh.rank][BUF_GATHER]);
@@ -1428,8 +1474,8 @@ int finish_step(vdjgraph_ctx *c, int step, bool device_barrier) {
     } else {
         CK(cudaStreamSynchronize(s));
     }
-    CK(cudaEventRecord(c->ev_fin[2 * step + 1], s));
-    sh.phase = 6 + step;
+    CK(cudaEventRecord(c->ev[EV_STEP0_MET + 2 * step], s));
+    sh.phase = finish_step_phase(step);
     return 0;
 }
 
@@ -1439,21 +1485,14 @@ int finish_end(vdjgraph_ctx *c) {
     Shard &sh = c->sh;
     cudaStream_t s = c->stream;
     vdjgraph_result &res = c->res;
-    Counters *d_ctr = c->d_ctr.as<Counters>();
     Counters *h_ctr = c->h_ctr.as<Counters>();
     const FinishLayout f = finish_layout(sh.surv_all, sh.G, sh.rank, c->prm.flags);
     int rc;
     res.hm_buckets = 0; res.ms_hashmap = 0;
     if (sh.rank == 0) {
-        const bool want_layout = c->prm.flags & VDJGRAPH_FLAG_HASHMAP_LAYOUT;
-        const bool want_keys = (c->prm.flags & VDJGRAPH_FLAG_EXPORT_KEYS) || want_layout;
         if (f.n_total) {
-            ExportArgs ae;
-            ae.table = nullptr; ae.cap = 0; ae.keys = nullptr; ae.vals = nullptr; ae.n = f.n_total;
-            ae.first_pos = c->d_first_pos.as<u64>(); ae.frequency = c->d_freq.as<u16>();
-            ae.out_deg = c->d_odeg.as<u8>(); ae.in_deg = c->d_ideg.as<u8>();
-            ae.out_succ = c->d_osucc.as<u32>(); ae.in_pred = c->d_ipred.as<u32>();
-            ae.kmer_lo = want_keys ? c->d_klo.as<u64>() : nullptr; ae.kmer_hi = want_keys ? c->d_khi.as<u64>() : nullptr;
+            ExportArgs ae = c->nodes.export_args(want_keys(c->prm.flags));
+            ae.n = f.n_total;
             const RowSink sink = row_sink(c->d_gather.as<char>(), f, c->prm.flags);
             k_unpack_rows<<<(int)((f.n_total + THREADS - 1) / THREADS), THREADS, 0, s>>>(sink, f.n_total, ae);
             k_unpack_overflow<<<c->sm_count, THREADS, 0, s>>>(sink, ae);
@@ -1461,17 +1500,15 @@ int finish_end(vdjgraph_ctx *c) {
             res.kernel_launches++;
             CK(cudaGetLastError());
         }
-        if (want_layout) {
+        if (c->prm.flags & VDJGRAPH_FLAG_HASHMAP_LAYOUT) {
             /* a peer that never arrived must not send the layout into a loop over garbage keys */
-            CK(cudaMemcpyAsync(h_ctr, d_ctr, sizeof(Counters), cudaMemcpyDeviceToHost, s));
-            CK(cudaStreamSynchronize(s));
+            if ((rc = read_counters(c))) return rc;
             if (h_ctr->internal) return fail(VDJGRAPH_ERR_INTERNAL, "sharded finish failed (code %u)", h_ctr->internal);
             if ((rc = run_hashmap_layout(c, f.n_total))) return rc;
         }
     }
-    CK(cudaEventRecord(c->ev[8], s));
-    CK(cudaMemcpyAsync(h_ctr, d_ctr, sizeof(Counters), cudaMemcpyDeviceToHost, s));
-    CK(cudaStreamSynchronize(s));
+    CK(cudaEventRecord(c->ev[EV_FINISH_END], s));
+    if ((rc = read_counters(c))) return rc;
     if (h_ctr->overflow) return fail(VDJGRAPH_ERR_INTERNAL, "survivor table overflow (code %u)", h_ctr->overflow);
     if (h_ctr->internal == 9) return fail(VDJGRAPH_ERR_INTERNAL, "a peer device did not reach the barrier of the sharded finish");
     if (h_ctr->internal) return fail(VDJGRAPH_ERR_INTERNAL, "export invariant violated (code %u)", h_ctr->internal);
@@ -1479,23 +1516,19 @@ int finish_end(vdjgraph_ctx *c) {
         return fail(VDJGRAPH_ERR_INTERNAL, "collected %llu nodes, expected %llu", (unsigned long long)h_ctr->n_nodes,
                     (unsigned long long)sh.surv_all[sh.rank]);
     c->ctr = *h_ctr;
-    if (res.hm_buckets) cudaEventElapsedTime(&res.ms_hashmap, c->ev_hm[0], c->ev_hm[1]);
-    res.ms_scatter = sh.acc[0]; res.ms_init1 = sh.acc[1]; res.ms_pass1 = sh.acc[2];
-    res.ms_prune = sh.acc[3]; res.ms_table2 = sh.acc[4]; res.ms_pass2 = sh.acc[5];
-    cudaEventElapsedTime(&res.ms_export, c->ev[12], c->ev[8]);
+    take_times(c);
     if (env_double("VDJGRAPH_FINISH_TIMES", 0) > 0) {
         /* where a distributed finish spends its time on this device: the three steps, the wait at the barrier
          * behind each, and (finishing device) unpacking the rows */
         float t[7];
-        cudaEvent_t seq[8] = { c->ev[12], c->ev_fin[0], c->ev_fin[1], c->ev_fin[2], c->ev_fin[3], c->ev_fin[4], c->ev_fin[5], c->ev[8] };
-        for (int i = 0; i < 7; i++) cudaEventElapsedTime(&t[i], seq[i], seq[i + 1]);
+        for (int i = 0; i < 7; i++) cudaEventElapsedTime(&t[i], c->ev[EV_FINISH + i], c->ev[EV_FINISH + i + 1]);
         fprintf(stderr, "vdjgraph finish rank %d: table+sort %.3f wait %.3f | rank %.3f wait %.3f | edges+rows %.3f wait %.3f | unpack %.3f ms\n",
                 sh.rank, t[0], t[1], t[2], t[3], t[4], t[5], t[6]);
     }
     res.ms_device = res.ms_scatter + res.ms_init1 + res.ms_pass1 + res.ms_prune + res.ms_table2 + res.ms_pass2 + res.ms_export;
     res.n_nodes = sh.rank == 0 ? f.n_total : 0;
     if (sh.rank == 0) res.n_pre = f.n_total;   /* (the other ranks keep their own survivor count) */
-    sh.phase = 9;
+    sh.phase = Phase::FINISHED;
     c->ran = sh.rank == 0;
     return 0;
 }
@@ -1534,10 +1567,7 @@ static int shard_stage_impl(vdjgraph_ctx *c, const char *primary, size_t np, con
         return fail(VDJGRAPH_ERR_PARAM, "record range exceeds total_records");
     if (info->total_records > 0xFFFFFFFEull)
         return fail(VDJGRAPH_ERR_TOO_MANY_NODES, "%llu records exceed the 2^32-2 record limit", (unsigned long long)info->total_records);
-    {
-        DevBuf *ex[NBUF] = { &c->d_bases, &c->d_valid, &c->d_qual, &c->d_strand, &c->d_tuples, &c->d_gather };
-        for (DevBuf *b : ex) b->exported = G > 1;
-    }
+    for (DevBuf *b : c->peer_bufs()) b->exported = G > 1;
     int rc = stage_impl(c, primary, np, secondary, ns, fwd);
     if (rc) return rc;
     Shard &sh = c->sh;
@@ -1562,20 +1592,20 @@ extern "C" int vdjgraph_shard_stage_forward(vdjgraph_ctx *c, const char *primary
 
 /* the per-bucket counts and HyperLogLog registers of this rank's staged records (k_count ran with the staging) */
 extern "C" int vdjgraph_shard_count(vdjgraph_ctx *c, uint64_t *hist, uint8_t *hll) {
-    if (c && c->staged && c->sh.phase == 9) c->sh.phase = 0;   /* another build of the same staged records */
-    int rc = phase_check(c, 0, "vdjgraph_shard_count");
+    if (c && c->staged && c->sh.phase == Phase::FINISHED) c->sh.phase = Phase::STAGED;   /* another build of the same staged records */
+    int rc = phase_check(c, Phase::STAGED, "vdjgraph_shard_count");
     if (rc) return rc;
     if (!hist || !hll) return fail(VDJGRAPH_ERR_PARAM, "NULL argument");
     c->ran = false;
     memcpy(hist, c->h_hist.p, HIST_WORDS * sizeof(uint64_t));
     memcpy(hll, c->h_hll.p, HLL_BYTES);
-    c->sh.phase = 1;
+    c->sh.phase = Phase::COUNTED;
     return 0;
 }
 
 extern "C" int vdjgraph_shard_plan(vdjgraph_ctx *c, const uint64_t *hist_all, const uint8_t *hll_merged,
                                    const uint64_t *record_counts) {
-    int rc = phase_check(c, 1, "vdjgraph_shard_plan");
+    int rc = phase_check(c, Phase::COUNTED, "vdjgraph_shard_plan");
     if (rc) return rc;
     if (!hist_all || !hll_merged || !record_counts) return fail(VDJGRAPH_ERR_PARAM, "NULL argument");
     CK(cudaSetDevice(c->device));
@@ -1601,32 +1631,31 @@ extern "C" int vdjgraph_shard_buffers(vdjgraph_ctx *c, void **ptrs, size_t *byte
 
 extern "C" int vdjgraph_shard_set_peers(vdjgraph_ctx *c, void *const *ptrs) {
     if (!c || !ptrs) return fail(VDJGRAPH_ERR_PARAM, "NULL argument");
-    if (c->sh.phase < 2) return fail(VDJGRAPH_ERR_STATE, "vdjgraph_shard_set_peers before vdjgraph_shard_plan");
+    if (c->sh.phase < Phase::PLANNED) return fail(VDJGRAPH_ERR_STATE, "vdjgraph_shard_set_peers before vdjgraph_shard_plan");
     Shard &sh = c->sh;
     for (int d = 0; d < sh.G; d++)
         for (int i = 0; i < NBUF; i++) sh.peer[d][i] = ptrs[d * NBUF + i];
-    own_buffers(c, sh.peer[sh.rank], nullptr);
-    sh.peers_set = true;
+    set_self_peers(c);
     return 0;
 }
 
 extern "C" int vdjgraph_shard_rounds(vdjgraph_ctx *c) {
     if (!c) return fail(VDJGRAPH_ERR_PARAM, "ctx is NULL");
-    if (!c->staged || c->sh.phase < 2) return fail(VDJGRAPH_ERR_STATE, "vdjgraph_shard_rounds before vdjgraph_shard_plan");
+    if (!c->staged || c->sh.phase < Phase::PLANNED) return fail(VDJGRAPH_ERR_STATE, "vdjgraph_shard_rounds before vdjgraph_shard_plan");
     return c->sh.S;
 }
 
 extern "C" int vdjgraph_shard_scatter(vdjgraph_ctx *c) {
     /* after the passes of a round that was not the last: the next round */
-    if (c && c->staged && c->sh.phase == 4 && c->sh.rnd + 1 < c->sh.S) { c->sh.rnd++; c->sh.phase = 2; }
-    int rc = phase_check(c, 2, "vdjgraph_shard_scatter");
+    if (c && c->staged && c->sh.phase == Phase::PASSES_DONE && c->sh.rnd + 1 < c->sh.S) { c->sh.rnd++; c->sh.phase = Phase::PLANNED; }
+    int rc = phase_check(c, Phase::PLANNED, "vdjgraph_shard_scatter");
     if (rc) return rc;
     CK(cudaSetDevice(c->device));
     return run_scatter(c);
 }
 
 extern "C" int vdjgraph_shard_passes(vdjgraph_ctx *c, uint64_t *n_survivors) {
-    int rc = phase_check(c, 3, "vdjgraph_shard_passes");
+    int rc = phase_check(c, Phase::SCATTERED, "vdjgraph_shard_passes");
     if (rc) return rc;
     CK(cudaSetDevice(c->device));
     if ((rc = run_passes(c))) return rc;
@@ -1636,7 +1665,7 @@ extern "C" int vdjgraph_shard_passes(vdjgraph_ctx *c, uint64_t *n_survivors) {
 }
 
 extern "C" int vdjgraph_shard_gather_plan(vdjgraph_ctx *c, const uint64_t *survivors_all) {
-    int rc = phase_check(c, 4, "vdjgraph_shard_gather_plan");
+    int rc = phase_check(c, Phase::PASSES_DONE, "vdjgraph_shard_gather_plan");
     if (rc) return rc;
     if (!survivors_all) return fail(VDJGRAPH_ERR_PARAM, "NULL argument");
     if (c->sh.rnd + 1 < c->sh.S)
@@ -1649,7 +1678,7 @@ extern "C" int vdjgraph_shard_gather_plan(vdjgraph_ctx *c, const uint64_t *survi
     for (int d = 0; d < sh.G; d++) { sh.surv_all[d] = survivors_all[d]; sh.surv_off[d] = off; off += survivors_all[d]; }
     sh.surv_off[sh.G] = off;
     if (sh.G > 1 && (rc = finish_plan(c))) return rc;
-    sh.phase = 5;
+    sh.phase = Phase::FINISH_PLANNED;
     return 0;
 }
 
@@ -1661,15 +1690,15 @@ extern "C" int vdjgraph_shard_finish_bytes(vdjgraph_ctx *c, const uint64_t *surv
 
 extern "C" int vdjgraph_shard_finish_step(vdjgraph_ctx *c, int step, int device_barrier) {
     if (step < 0 || step > 2) return fail(VDJGRAPH_ERR_PARAM, "finish step %d", step);
-    int rc = phase_check(c, 5 + step, "vdjgraph_shard_finish_step");
+    int rc = phase_check(c, step ? finish_step_phase(step - 1) : Phase::FINISH_PLANNED, "vdjgraph_shard_finish_step");
     if (rc) return rc;
     CK(cudaSetDevice(c->device));
-    if (c->sh.G == 1) { c->sh.phase = 6 + step; return 0; }   /* one device: everything happens in vdjgraph_shard_finish */
+    if (c->sh.G == 1) { c->sh.phase = finish_step_phase(step); return 0; }   /* one device: everything happens in vdjgraph_shard_finish */
     return finish_step(c, step, device_barrier != 0);
 }
 
 extern "C" int vdjgraph_shard_finish(vdjgraph_ctx *c) {
-    int rc = phase_check(c, 8, "vdjgraph_shard_finish");
+    int rc = phase_check(c, Phase::FINISH_STEP2, "vdjgraph_shard_finish");
     if (rc) return rc;
     CK(cudaSetDevice(c->device));
     return c->sh.G == 1 ? run_finish(c) : finish_end(c);
@@ -1680,8 +1709,7 @@ extern "C" int vdjgraph_shard_finish(vdjgraph_ctx *c) {
 extern "C" int vdjgraph_shard_release_retired(vdjgraph_ctx *c) {
     if (!c) return fail(VDJGRAPH_ERR_PARAM, "ctx is NULL");
     CK(cudaSetDevice(c->device));
-    DevBuf *ex[NBUF] = { &c->d_bases, &c->d_valid, &c->d_qual, &c->d_strand, &c->d_tuples, &c->d_gather };
-    for (DevBuf *b : ex) b->release_retired();
+    for (DevBuf *b : c->peer_bufs()) b->release_retired();
     return 0;
 }
 
@@ -1750,31 +1778,10 @@ extern "C" int vdjgraph_fetch(vdjgraph_ctx *c, vdjgraph_result *out) {
     if (!c->ran) return fail(VDJGRAPH_ERR_STATE, "vdjgraph_fetch before vdjgraph_run");
     CK(cudaSetDevice(c->device));
     double t0 = wall_ms();
-    const uint64_t n = c->res.n_nodes;
-    const size_t na = std::max<uint64_t>(n, 1);
-    const bool want_keys = c->prm.flags & VDJGRAPH_FLAG_EXPORT_KEYS;
-    int rc;
-    if ((rc = c->h_first_pos.ensure(na * 8)) || (rc = c->h_freq.ensure(na * 2)) || (rc = c->h_odeg.ensure(na)) ||
-        (rc = c->h_ideg.ensure(na)) || (rc = c->h_osucc.ensure(na * 16)) || (rc = c->h_ipred.ensure(na * 16)))
-        return rc;
-    if (want_keys && ((rc = c->h_klo.ensure(na * 8)) || (rc = c->h_khi.ensure(na * 8)))) return rc;
+    vdjgraph_result &r = c->res;
     uint64_t bytes = 0;
-    if (n) {
-        cudaStream_t s = c->stream;
-        CK(cudaMemcpyAsync(c->h_first_pos.p, c->d_first_pos.p, n * 8, cudaMemcpyDeviceToHost, s));
-        CK(cudaMemcpyAsync(c->h_freq.p, c->d_freq.p, n * 2, cudaMemcpyDeviceToHost, s));
-        CK(cudaMemcpyAsync(c->h_odeg.p, c->d_odeg.p, n, cudaMemcpyDeviceToHost, s));
-        CK(cudaMemcpyAsync(c->h_ideg.p, c->d_ideg.p, n, cudaMemcpyDeviceToHost, s));
-        CK(cudaMemcpyAsync(c->h_osucc.p, c->d_osucc.p, n * 16, cudaMemcpyDeviceToHost, s));
-        CK(cudaMemcpyAsync(c->h_ipred.p, c->d_ipred.p, n * 16, cudaMemcpyDeviceToHost, s));
-        bytes = n * (8 + 2 + 1 + 1 + 16 + 16);
-        if (want_keys) {
-            CK(cudaMemcpyAsync(c->h_klo.p, c->d_klo.p, n * 8, cudaMemcpyDeviceToHost, s));
-            CK(cudaMemcpyAsync(c->h_khi.p, c->d_khi.p, n * 8, cudaMemcpyDeviceToHost, s));
-            bytes += n * 16;
-        }
-        CK(cudaStreamSynchronize(s));
-    }
+    int rc;
+    if ((rc = c->nodes.fetch(r.n_nodes, c->prm.flags & VDJGRAPH_FLAG_EXPORT_KEYS, c->stream, r, bytes))) return rc;
     if (c->res.hm_buckets) {   /* the layout exists even for an empty graph: 32 empty buckets */
         cudaStream_t s = c->stream;
         if ((rc = c->h_hm_slots.ensure(c->res.hm_buckets * 4))) return rc;
@@ -1782,16 +1789,7 @@ extern "C" int vdjgraph_fetch(vdjgraph_ctx *c, vdjgraph_result *out) {
         CK(cudaStreamSynchronize(s));
         bytes += c->res.hm_buckets * 4;
     }
-    vdjgraph_result &r = c->res;
     r.hm_slots = c->res.hm_buckets ? c->h_hm_slots.as<uint32_t>() : nullptr;
-    r.first_pos = c->h_first_pos.as<uint64_t>();
-    r.frequency = c->h_freq.as<uint16_t>();
-    r.out_deg = c->h_odeg.as<uint8_t>();
-    r.in_deg = c->h_ideg.as<uint8_t>();
-    r.out_succ = c->h_osucc.as<uint32_t>();
-    r.in_pred = c->h_ipred.as<uint32_t>();
-    r.kmer_lo = want_keys ? c->h_klo.as<uint64_t>() : nullptr;
-    r.kmer_hi = want_keys ? c->h_khi.as<uint64_t>() : nullptr;
     r.d2h_bytes = bytes;
     r.ms_fetch = (float)(wall_ms() - t0);
     *out = r;
@@ -1800,7 +1798,7 @@ extern "C" int vdjgraph_fetch(vdjgraph_ctx *c, vdjgraph_result *out) {
 
 extern "C" int vdjgraph_stats(vdjgraph_ctx *c, vdjgraph_result *out) {
     if (!c || !out) return fail(VDJGRAPH_ERR_PARAM, "NULL argument");
-    if (!c->ran && c->sh.phase < 9) return fail(VDJGRAPH_ERR_STATE, "vdjgraph_stats before vdjgraph_run");
+    if (!c->ran && c->sh.phase < Phase::FINISHED) return fail(VDJGRAPH_ERR_STATE, "vdjgraph_stats before vdjgraph_run");
     *out = c->res;
     out->first_pos = nullptr; out->frequency = nullptr; out->out_deg = out->in_deg = nullptr;
     out->out_succ = out->in_pred = nullptr; out->kmer_lo = out->kmer_hi = nullptr; out->hm_slots = nullptr;
