@@ -302,6 +302,37 @@ int vdjgraph_stats(vdjgraph_ctx *ctx, vdjgraph_result *out);
 /* Parity/debug: the pruned pass-1 table of the last run. */
 int vdjgraph_fetch_pre_table(vdjgraph_ctx *ctx, vdjgraph_pre_table *out);
 
+/*
+ * Look sequences up in the graph of the last finished vdjgraph_run / vdjgraph_build / _forward on this
+ * context: which node is the k-mer of every window, and where along a sequence does the graph break.
+ * The lookups run on the device against the graph's own survivor table.
+ *
+ * Query i is seqs[offsets[i] .. offsets[i+1]); offsets must not decrease (offsets may be NULL when
+ * n_queries is 0).  Its windows are the k-mers starting at bytes 0 .. len-k; a query shorter than k has
+ * none.  The alphabet is the staging alphabet: an N ends the windows over it, as in a read, and any
+ * other byte outside ACGT (lower case included) fails the call with VDJGRAPH_ERR_BASE.  n_windows must
+ * be the exact window count, sum over queries of max(0, len - k + 1), or the call fails with
+ * VDJGRAPH_ERR_PARAM.  On any failure node_of_window is not written.
+ *
+ * VDJGRAPH_ERR_STATE: no run has finished since the context was created or since the last
+ * vdjgraph_stage* / vdjgraph_set_params / vdjgraph_shard_stage*, or the last build ran the sharded
+ * phases over more than one rank (each rank's table holds its own share only).
+ * Synchronous, on the context's stream; the graph and what vdjgraph_fetch returns are unchanged.
+ */
+typedef struct vdjgraph_query_stats {
+    uint64_t n_queries, n_windows;   /* windows = sum over queries of max(0, len - k + 1) */
+    uint64_t n_found;                /* windows whose k-mer is a node */
+    uint64_t h2d_bytes, d2h_bytes;
+    float ms_kernels;                /* CUDA events around the query kernels */
+    float ms_total;                  /* wall clock of the call */
+} vdjgraph_query_stats;
+
+/* node (creation rank, = reference id - 1) of every k-mer window of every query, in query order;
+ * 0xFFFFFFFF where the window holds an N or its k-mer is not a node */
+int vdjgraph_query(vdjgraph_ctx *ctx, const char *seqs, const uint64_t *offsets /*[n_queries+1]*/,
+                   size_t n_queries, uint32_t *node_of_window, size_t n_windows,
+                   vdjgraph_query_stats *stats /* may be NULL */);
+
 #ifdef __cplusplus
 }
 #endif

@@ -5,7 +5,7 @@ libvdjgraph.so).  The library replaces the block assembler2_vdj.c:1381-1415 of t
 (build_pre_graph x2 -> prune_pre_graph -> build_graph2 x2); there is no CPU fallback here:
 importing works anywhere, but creating a GraphBuilder without the CUDA library or a B200 raises.
 """
-from .graph import GraphBuilder, MultiBuilder, Graph, PinnedRecords, PreTable, VdjGraphError, forward_reads, host_alloc, host_free, lib_path  # noqa: F401
+from .graph import GraphBuilder, MultiBuilder, Graph, PinnedRecords, PreTable, VdjGraphError, forward_reads, host_alloc, host_free, lib_path, NIL, query_batch, window_counts  # noqa: F401
 from . import synth  # noqa: F401
 
-__all__ = ["GraphBuilder", "MultiBuilder", "Graph", "PinnedRecords", "PreTable", "VdjGraphError", "forward_reads", "host_alloc", "host_free", "lib_path", "synth"]
+__all__ = ["GraphBuilder", "MultiBuilder", "Graph", "PinnedRecords", "PreTable", "VdjGraphError", "forward_reads", "host_alloc", "host_free", "lib_path", "NIL", "query_batch", "window_counts", "synth"]

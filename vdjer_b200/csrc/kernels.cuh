@@ -2250,4 +2250,109 @@ k_export_pre(const Slot1 *t, u64 cap, u64 *klo, u64 *khi, u16 *freq, u64 *n_out)
     }
 }
 
+/* ------------------------------------------------------------------------------------------ */
+/* Queries (vdjgraph_query): the node of every k-mer window of caller sequences, looked up in the */
+/* finished survivor table (rank in the upper half of word 2, as k_export reads it).  The host     */
+/* streams the batch in chunks of whole queries; per chunk k_query_pack packs the text and        */
+/* k_query answers its windows.                                                                    */
+/* ------------------------------------------------------------------------------------------ */
+/* One thread per 64 bytes of the chunk's text: 2-bit bases (A0 C1 G2 T3, N stored as 0, base j at bits
+ * 2j of the chunk's words: the key layout) and a mask, bit j = byte j is not ACGT.  A byte outside ACGTN
+ * lowers bad[0] to its position in the batch (base + j), as staging flags a bad base.  The text buffer is
+ * readable up to the next multiple of 64 bytes; bytes past n are ignored. */
+__global__ void __launch_bounds__(THREADS)
+k_query_pack(const unsigned char *text, u64 n, u64 base, u64 *bases, u64 *nmask, u64 *bad) {
+    const u64 t = (u64)blockIdx.x * blockDim.x + threadIdx.x;
+    const u64 j0 = t * 64;
+    if (j0 >= n) return;
+    const uint4 *src = reinterpret_cast<const uint4 *>(text + j0);
+    u64 b[2] = { 0, 0 }, nm = 0, first_bad = ~0ull;
+#pragma unroll
+    for (int q = 0; q < 4; q++) {
+        const uint4 v = src[q];
+        const u32 words[4] = { v.x, v.y, v.z, v.w };
+#pragma unroll
+        for (int j = 16 * q; j < 16 * q + 16; j++) {
+            const u32 ch = (words[(j >> 2) & 3] >> (8 * (j & 3))) & 0xFFu;
+            const u32 code = ch == 'C' ? 1u : ch == 'G' ? 2u : ch == 'T' ? 3u : 0u;
+            const bool acgt = code != 0u || ch == 'A';
+            b[j >> 5] |= (u64)code << (2 * (j & 31));
+            if (!acgt && j0 + j < n) {
+                nm |= 1ull << j;
+                if (ch != 'N') first_bad = min(first_bad, j0 + j);
+            }
+        }
+    }
+    bases[2 * t] = b[0];
+    bases[2 * t + 1] = b[1];
+    nmask[t] = nm;
+    if (first_bad != ~0ull) atomicMin(bad, base + first_bad);
+}
+
+struct QueryArgs {
+    const u64 *bases, *nmask;   /* k_query_pack's output for the chunk */
+    u64 n_words, n_mwords;      /* their lengths in words */
+    const u64 *qoff;            /* [nq] first byte of query i in the chunk */
+    const u64 *woff;            /* [nq + 1] first window of query i in the chunk; woff[nq] = nw */
+    u64 nq, nw;
+    const Slot2 *table;         /* the finished survivor table; null when the graph has no nodes */
+    u64 cap;
+    u32 *out;                   /* [nw] creation rank, NIL32 = N in the window or not a node */
+    u64 *found;                 /* += windows whose k-mer is a node (one atomic per warp) */
+};
+
+/* BATCH consecutive windows per thread: their first probes are issued back to back (the table is far
+ * larger than L2 on real inputs, every probe is a random HBM sector); the rare longer probe sequences
+ * continue one by one.  The query of the first window is found by binary search over woff, the others
+ * by stepping forward. */
+__global__ void __launch_bounds__(THREADS)
+k_query(QueryArgs a, Geom g, Part pt) {
+    const u64 w0 = ((u64)blockIdx.x * blockDim.x + threadIdx.x) * BATCH;
+    u32 n_found = 0;
+    if (w0 < a.nw) {
+        u64 l = 0, r = a.nq;   /* woff[l] <= w0 < woff[r] */
+        while (r - l > 1) {
+            const u64 m = (l + r) >> 1;
+            if (a.woff[m] <= w0) l = m; else r = m;
+        }
+        u64 q = l, cur = a.woff[q], next = a.woff[q + 1];
+        u64 lo[BATCH], hi[BATCH], idx[BATCH], q2[BATCH], q3[BATCH];
+        bool live[BATCH];
+        u32 rank[BATCH];
+#pragma unroll
+        for (int b = 0; b < BATCH; b++) {
+            const u64 w = w0 + b;
+            live[b] = false; rank[b] = NIL32; lo[b] = hi[b] = 0; idx[b] = 0;
+            if (w >= a.nw) continue;
+            while (w >= next) { q++; cur = next; next = a.woff[q + 1]; }
+            const u64 p = a.qoff[q] + (w - cur);   /* first byte of the window in the chunk */
+            const u64 mw = p >> 6, bw = p >> 5;
+            if (extract_mask(a.nmask + mw, (int)min((u64)2, a.n_mwords - mw), (int)(p & 63)) & g.kones) continue;
+            extract_kmer(a.bases + bw, (int)min((u64)3, a.n_words - bw), (int)(p & 31), g.kmask_lo, g.kmask_hi, lo[b], hi[b]);
+            if (!a.table) continue;
+            idx[b] = t2_home(pt, g, lo[b], hi[b]);
+            live[b] = true;
+        }
+        u64 k0[BATCH], k1[BATCH];
+#pragma unroll
+        for (int b = 0; b < BATCH; b++)
+            if (live[b]) ld_sector(&a.table[idx[b]], k0[b], k1[b], q2[b], q3[b]);
+#pragma unroll
+        for (int b = 0; b < BATCH; b++) {
+            if (!live[b]) continue;
+            bool hit = k0[b] == lo[b] && k1[b] == hi[b];
+            if (!hit && !(k0[b] == EMPTY64 && k1[b] == EMPTY64)) {
+                const u64 from = idx[b] + 1 == a.cap ? 0 : idx[b] + 1;
+                hit = t2_probe_from(a.table, a.cap, from, lo[b], hi[b], q2[b], q3[b]) != INF64;
+            }
+            if (hit) { rank[b] = (u32)(q2[b] >> 32); n_found++; }
+        }
+#pragma unroll
+        for (int b = 0; b < BATCH; b++)
+            if (w0 + b < a.nw) a.out[w0 + b] = rank[b];
+    }
+    n_found = __reduce_add_sync(0xFFFFFFFFu, n_found);
+    if ((threadIdx.x & 31) == 0 && n_found) atomicAdd(a.found, (u64)n_found);
+}
+
 } // namespace vdjg

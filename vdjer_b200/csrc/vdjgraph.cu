@@ -204,7 +204,48 @@ enum Ev {
 };
 static_assert(EV_FINISH_END == EV_FINISH + 7, "the finish's events are consecutive");
 
+/* The finished graph's survivor table as vdjgraph_query looks k-mers up in it: the table k_export read
+ * (one round: d_t2 with the per-unit slices of the plan; several rounds: the merged flat table d_t2m)
+ * and the slicing and geometry it was read with.  Valid from the end of a one-device finish until the
+ * next stage, set_params or run; table is null when the graph has no nodes. */
+struct GraphView {
+    bool valid = false;
+    const Slot2 *table = nullptr;
+    uint64_t cap = 0, n_nodes = 0;
+    Part pt{};
+    Geom g{};
+};
+
+/* vdjgraph_query's buffers: chunks of the batch go through page-locked text and offset buffers, are
+ * copied on their own stream (h2d) and answered on the context's stream, double buffered: the next
+ * chunk's copy overlaps the current chunk's kernels.  The answers of the whole batch stay on the device
+ * until every chunk has passed the alphabet check. */
+struct QueryBufs {
+    cudaStream_t h2d = nullptr;
+    cudaEvent_t copied[2] = {}, k_begin[2] = {}, k_end[2] = {};
+    bool pending[2] = { false, false };  /* chunk kernels queued behind k_end[b] whose time is not yet added */
+    PinBuf text[2], meta[2], ctr;
+    DevBuf d_text[2], d_meta[2], d_bases, d_nmask, d_out, d_ctr;
+    int init() {
+        if (h2d) return 0;
+        CK(cudaStreamCreateWithFlags(&h2d, cudaStreamNonBlocking));
+        for (int b = 0; b < 2; b++) {
+            CK(cudaEventCreateWithFlags(&copied[b], cudaEventDisableTiming));
+            CK(cudaEventCreate(&k_begin[b]));
+            CK(cudaEventCreate(&k_end[b]));
+        }
+        return 0;
+    }
+    void destroy() {
+        for (int b = 0; b < 2; b++)
+            for (cudaEvent_t e : { copied[b], k_begin[b], k_end[b] }) if (e) cudaEventDestroy(e);
+        if (h2d) cudaStreamDestroy(h2d);
+        h2d = nullptr;
+    }
+};
+
 constexpr uint32_t STAGE_CHUNK = 32768; /* records per staging chunk (3.3 MB of text at L=50) */
+constexpr size_t QUERY_CHUNK = 32ull << 20;   /* bytes of query text per chunk (VDJGRAPH_QUERY_CHUNK_KB overrides) */
 constexpr double MERGED_SLOTS_PER_NODE = 2.0;   /* slots of the merged survivor table per node (load 0.5) */
 constexpr uint64_t REF_MAX_NODES = 900000000ull; /* MAX_NODES, assembler2_vdj.c:73 */
 constexpr uint64_t SLICE_BYTES = 12ull << 20;   /* table-1 bytes one hash unit addresses: L2-resident (12 MB measured better than 24 and 6) */
@@ -286,6 +327,9 @@ struct vdjgraph_ctx {
     uint32_t log_cap = 0;
     Counters ctr;
     vdjgraph_result res;
+
+    GraphView view;   /* what vdjgraph_query looks k-mers up in */
+    QueryBufs q;
 };
 
 namespace {
@@ -567,6 +611,7 @@ extern "C" void vdjgraph_destroy(vdjgraph_ctx *c) {
         if (w.stream) cudaStreamDestroy(w.stream);
     }
     for (cudaEvent_t ev : c->ev) if (ev) cudaEventDestroy(ev);
+    c->q.destroy();
     if (c->stream) cudaStreamDestroy(c->stream);
     delete c;   /* the buffers free themselves */
 }
@@ -580,7 +625,7 @@ extern "C" int vdjgraph_set_params(vdjgraph_ctx *c, const vdjgraph_params *param
     c->prm = *params;
     c->prm.device = dev;
     if (regeom) { c->staged = false; }
-    c->ran = false;
+    c->ran = false; c->view.valid = false;
     return 0;
 }
 
@@ -593,7 +638,7 @@ static int stage_impl(vdjgraph_ctx *c, const char *primary, size_t np, const cha
     if (!c) return fail(VDJGRAPH_ERR_PARAM, "ctx is NULL");
     if ((np && !primary) || (ns && !secondary)) return fail(VDJGRAPH_ERR_PARAM, "NULL record buffer");
     CK(cudaSetDevice(c->device));
-    c->staged = false; c->ran = false;
+    c->staged = false; c->ran = false; c->view.valid = false;
     const uint64_t Rt = (uint64_t)np + (uint64_t)ns;   /* text records */
     const uint64_t R = Rt << fwd;                      /* packed records */
     if (R > 0xFFFFFFFEull) return fail(VDJGRAPH_ERR_TOO_MANY_NODES, "%llu records exceed the 2^32-2 record limit", (unsigned long long)R);
@@ -1339,6 +1384,9 @@ int run_finish(vdjgraph_ctx *c) {
     cudaEventElapsedTime(&res.ms_device, c->ev[EV_BUILD], c->ev[EV_FINISH_END]);
     sh.phase = Phase::FINISHED;
     c->ran = true;
+    c->view.table = n_surv ? table : nullptr;
+    c->view.cap = cap2; c->view.n_nodes = n_surv; c->view.pt = pt; c->view.g = g;
+    c->view.valid = true;
     return 0;
 }
 
@@ -1540,9 +1588,15 @@ extern "C" int vdjgraph_run(vdjgraph_ctx *c) {
     if (!c->staged) return fail(VDJGRAPH_ERR_STATE, "vdjgraph_run before vdjgraph_stage");
     if (c->sh.G != 1) return fail(VDJGRAPH_ERR_STATE, "vdjgraph_run on a sharded context; use the vdjgraph_shard_* phases");
     CK(cudaSetDevice(c->device));
-    c->ran = false;
+    c->ran = false; c->view.valid = false;
     int rc;
-    if (c->g.R == 0) { reset_run_stats(c); c->ran = true; return 0; }
+    if (c->g.R == 0) {
+        reset_run_stats(c);
+        c->ran = true;
+        c->view = GraphView();   /* no nodes: every window answers NIL */
+        c->view.g = c->g; c->view.valid = true;
+        return 0;
+    }
     if ((rc = run_plan(c, c->h_hist.as<uint64_t>(), c->h_hll.as<uint8_t>()))) return rc;
     set_self_peers(c);
     for (int r = 0; r < c->sh.S; r++) {
@@ -1596,7 +1650,7 @@ extern "C" int vdjgraph_shard_count(vdjgraph_ctx *c, uint64_t *hist, uint8_t *hl
     int rc = phase_check(c, Phase::STAGED, "vdjgraph_shard_count");
     if (rc) return rc;
     if (!hist || !hll) return fail(VDJGRAPH_ERR_PARAM, "NULL argument");
-    c->ran = false;
+    c->ran = false; c->view.valid = false;
     memcpy(hist, c->h_hist.p, HIST_WORDS * sizeof(uint64_t));
     memcpy(hll, c->h_hll.p, HLL_BYTES);
     c->sh.phase = Phase::COUNTED;
@@ -1850,6 +1904,149 @@ extern "C" int vdjgraph_fetch_pre_table(vdjgraph_ctx *c, vdjgraph_pre_table *out
     out->kmer_lo = c->h_pre_klo.as<uint64_t>();
     out->kmer_hi = c->h_pre_khi.as<uint64_t>();
     out->frequency = c->h_pre_freq.as<uint16_t>();
+    return 0;
+}
+
+/* ========================================================================================== */
+/* Queries: the node of every k-mer window of caller sequences (k_query_pack, k_query)          */
+/* ========================================================================================== */
+extern "C" int vdjgraph_query(vdjgraph_ctx *c, const char *seqs, const uint64_t *offsets, size_t nq,
+                              uint32_t *out, size_t n_windows, vdjgraph_query_stats *stats) {
+    const double t0 = wall_ms();
+    if (!c) return fail(VDJGRAPH_ERR_PARAM, "ctx is NULL");
+    if (!c->view.valid) {
+        if (c->sh.G > 1 && c->sh.phase == Phase::FINISHED)
+            return fail(VDJGRAPH_ERR_STATE, "vdjgraph_query on a graph built over %d ranks: each rank's table holds its own share", c->sh.G);
+        return fail(VDJGRAPH_ERR_STATE, "vdjgraph_query before vdjgraph_run (or after vdjgraph_stage / vdjgraph_set_params)");
+    }
+    if (nq && !offsets) return fail(VDJGRAPH_ERR_PARAM, "offsets is NULL");
+    const GraphView &v = c->view;
+    const uint64_t k = (uint64_t)v.g.k;
+    auto windows_of = [k](uint64_t len) { return len >= k ? len - k + 1 : 0; };
+    uint64_t total = 0;
+    for (size_t i = 0; i < nq; i++) {
+        if (offsets[i + 1] < offsets[i]) return fail(VDJGRAPH_ERR_PARAM, "offsets decrease at query %zu", i);
+        total += windows_of(offsets[i + 1] - offsets[i]);
+    }
+    if (total != n_windows)
+        return fail(VDJGRAPH_ERR_PARAM, "n_windows is %zu, the queries have %llu windows", n_windows, (unsigned long long)total);
+    const uint64_t t_lo = nq ? offsets[0] : 0, n_bytes = nq ? offsets[nq] - offsets[0] : 0;
+    if ((n_bytes && !seqs) || (n_windows && !out)) return fail(VDJGRAPH_ERR_PARAM, "NULL buffer");
+    CK(cudaSetDevice(c->device));
+    cudaStream_t s = c->stream;
+    QueryBufs &qb = c->q;
+    int rc;
+    if ((rc = qb.init())) return rc;
+    const double chunk_kb = env_double("VDJGRAPH_QUERY_CHUNK_KB", 0);
+    const uint64_t CH = chunk_kb > 0 ? std::max<uint64_t>(64, (uint64_t)(chunk_kb * 1024)) : QUERY_CHUNK;
+    const uint64_t QMAX = std::max<uint64_t>(1024, CH / 16);   /* queries per chunk (empty ones take no bytes) */
+    if ((rc = qb.d_ctr.ensure(16)) || (rc = qb.ctr.ensure(16)) || (rc = qb.d_out.ensure(std::max<size_t>(n_windows, 1) * 4)) ||
+        (rc = qb.d_bases.ensure(CH / 4 + 64)) || (rc = qb.d_nmask.ensure(CH / 8 + 64)))
+        return rc;
+    uint64_t *hc = qb.ctr.as<uint64_t>();   /* [0] windows found, [1] first byte outside ACGTN */
+    hc[0] = 0; hc[1] = ~0ull;
+    CK(cudaMemcpyAsync(qb.d_ctr.p, hc, 16, cudaMemcpyHostToDevice, s));
+    uint64_t h2d = 16, d2h = 0;
+    const bool direct = is_page_locked(seqs + t_lo, n_bytes);   /* page-locked text: DMA straight out of it */
+    float ms_kernels = 0;
+    qb.pending[0] = qb.pending[1] = false;
+    auto retire = [&](int b) -> int {   /* chunk kernels behind k_end[b] have finished: add their time */
+        if (!qb.pending[b]) return 0;
+        CK(cudaEventSynchronize(qb.k_end[b]));
+        float ms = 0;
+        CK(cudaEventElapsedTime(&ms, qb.k_begin[b], qb.k_end[b]));
+        ms_kernels += ms;
+        qb.pending[b] = false;
+        return 0;
+    };
+    /* chunks of whole queries, at most CH bytes unless one query alone is longer */
+    uint64_t w_base = 0;
+    for (uint64_t i = 0, chunk = 0; i < nq; chunk++) {
+        const int b = (int)(chunk & 1);
+        if ((rc = retire(b))) return rc;   /* the kernels of chunk - 2 are done with buffer set b */
+        const uint64_t c_lo = offsets[i];
+        uint64_t j = i + 1;
+        while (j < nq && j - i < QMAX && offsets[j + 1] - c_lo <= CH) j++;
+        const uint64_t nb = offsets[j] - c_lo, nqc = j - i, nb_pad = std::max<uint64_t>(64, (nb + 63) & ~63ull);
+        const size_t meta_bytes = (2 * nqc + 1) * sizeof(uint64_t);
+        if ((rc = qb.meta[b].ensure(meta_bytes)) || (rc = qb.d_meta[b].ensure(meta_bytes)) || (rc = qb.d_text[b].ensure(nb_pad)) ||
+            (rc = qb.d_bases.ensure(nb_pad / 4)) || (rc = qb.d_nmask.ensure(nb_pad / 8)) || (!direct && (rc = qb.text[b].ensure(nb))))
+            return rc;
+        uint64_t *qoff = qb.meta[b].as<uint64_t>(), *woff = qoff + nqc, wn = 0;
+        for (uint64_t x = 0; x < nqc; x++) {
+            qoff[x] = offsets[i + x] - c_lo;
+            woff[x] = wn;
+            wn += windows_of(offsets[i + x + 1] - offsets[i + x]);
+        }
+        woff[nqc] = wn;
+        const char *src = seqs + c_lo;
+        if (!direct && nb) { memcpy(qb.text[b].p, src, nb); src = qb.text[b].as<char>(); }
+        if (nb) CK(cudaMemcpyAsync(qb.d_text[b].p, src, nb, cudaMemcpyHostToDevice, qb.h2d));
+        CK(cudaMemcpyAsync(qb.d_meta[b].p, qoff, meta_bytes, cudaMemcpyHostToDevice, qb.h2d));
+        CK(cudaEventRecord(qb.copied[b], qb.h2d));
+        h2d += nb + meta_bytes;
+        CK(cudaStreamWaitEvent(s, qb.copied[b], 0));
+        CK(cudaEventRecord(qb.k_begin[b], s));
+        u64 *d_ctr = qb.d_ctr.as<u64>();
+        if (nb)
+            k_query_pack<<<(int)((nb_pad / 64 + THREADS - 1) / THREADS), THREADS, 0, s>>>(
+                qb.d_text[b].as<unsigned char>(), nb, c_lo - t_lo, qb.d_bases.as<u64>(), qb.d_nmask.as<u64>(), d_ctr + 1);
+        if (wn) {
+            QueryArgs qa;
+            qa.bases = qb.d_bases.as<u64>(); qa.nmask = qb.d_nmask.as<u64>();
+            qa.n_words = nb_pad / 32; qa.n_mwords = nb_pad / 64;
+            qa.qoff = qb.d_meta[b].as<u64>(); qa.woff = qa.qoff + nqc;
+            qa.nq = nqc; qa.nw = wn;
+            qa.table = v.table; qa.cap = v.cap;
+            qa.out = qb.d_out.as<u32>() + w_base;
+            qa.found = d_ctr;
+            const uint64_t per_block = (uint64_t)THREADS * BATCH;
+            k_query<<<(int)((wn + per_block - 1) / per_block), THREADS, 0, s>>>(qa, v.g, v.pt);
+        }
+        CK(cudaGetLastError());
+        CK(cudaEventRecord(qb.k_end[b], s));
+        qb.pending[b] = true;
+        w_base += wn;
+        i = j;
+    }
+    for (int b = 0; b < 2; b++) if ((rc = retire(b))) return rc;
+    CK(cudaMemcpyAsync(hc, qb.d_ctr.p, 16, cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    d2h += 16;
+    if (hc[1] != ~0ull) {
+        const uint64_t pos = t_lo + hc[1];
+        const size_t qi = (size_t)(std::upper_bound(offsets, offsets + nq + 1, pos) - offsets) - 1;
+        return fail(VDJGRAPH_ERR_BASE, "byte %llu of query %zu is outside ACGTN", (unsigned long long)(pos - offsets[qi]), qi);
+    }
+    /* every chunk passed the alphabet check: the answers to the caller (through page-locked chunks unless
+     * its array is page-locked itself) */
+    const uint64_t out_bytes = (uint64_t)n_windows * 4;
+    if (out_bytes && is_page_locked(out, out_bytes)) {
+        CK(cudaMemcpyAsync(out, qb.d_out.p, out_bytes, cudaMemcpyDeviceToHost, s));
+        CK(cudaStreamSynchronize(s));
+    } else if (out_bytes) {
+        if ((rc = qb.text[0].ensure(CH)) || (rc = qb.text[1].ensure(CH))) return rc;
+        const uint64_t n_parts = (out_bytes + CH - 1) / CH;
+        for (uint64_t part = 0; part <= n_parts; part++) {
+            if (part < n_parts) {   /* queue part, then hand over part - 1 while it copies */
+                const uint64_t o = part * CH;
+                CK(cudaMemcpyAsync(qb.text[part & 1].p, qb.d_out.as<char>() + o, std::min(CH, out_bytes - o), cudaMemcpyDeviceToHost, s));
+                CK(cudaEventRecord(qb.copied[part & 1], s));
+            }
+            if (part > 0) {
+                const uint64_t p = part - 1, o = p * CH;
+                CK(cudaEventSynchronize(qb.copied[p & 1]));
+                memcpy(reinterpret_cast<char *>(out) + o, qb.text[p & 1].p, std::min(CH, out_bytes - o));
+            }
+        }
+    }
+    d2h += out_bytes;
+    if (stats) {
+        stats->n_queries = nq; stats->n_windows = n_windows; stats->n_found = hc[0];
+        stats->h2d_bytes = h2d; stats->d2h_bytes = d2h;
+        stats->ms_kernels = ms_kernels;
+        stats->ms_total = (float)(wall_ms() - t0);
+    }
     return 0;
 }
 

@@ -56,6 +56,11 @@ class _Result(C.Structure):
     ]
 
 
+class _QueryStats(C.Structure):
+    _fields_ = [("n_queries", C.c_uint64), ("n_windows", C.c_uint64), ("n_found", C.c_uint64),
+                ("h2d_bytes", C.c_uint64), ("d2h_bytes", C.c_uint64), ("ms_kernels", C.c_float), ("ms_total", C.c_float)]
+
+
 class _PreTable(C.Structure):
     _fields_ = [("n", C.c_uint64), ("kmer_lo", C.POINTER(C.c_uint64)),
                 ("kmer_hi", C.POINTER(C.c_uint64)), ("frequency", C.POINTER(C.c_uint16))]
@@ -69,7 +74,7 @@ EXPORTS = [
     "vdjgraph_version", "vdjgraph_last_error", "vdjgraph_create", "vdjgraph_destroy",
     "vdjgraph_set_params", "vdjgraph_build", "vdjgraph_stage", "vdjgraph_run", "vdjgraph_fetch",
     "vdjgraph_stage_forward", "vdjgraph_build_forward",
-    "vdjgraph_fetch_pre_table", "vdjgraph_stats",
+    "vdjgraph_fetch_pre_table", "vdjgraph_stats", "vdjgraph_query",
     "vdjgraph_host_alloc", "vdjgraph_host_free", "vdjgraph_host_register", "vdjgraph_host_unregister",
     "vdjgraph_shard_stage", "vdjgraph_shard_stage_forward", "vdjgraph_shard_count", "vdjgraph_shard_plan", "vdjgraph_shard_rounds", "vdjgraph_shard_buffers",
     "vdjgraph_shard_set_peers", "vdjgraph_shard_scatter", "vdjgraph_shard_passes", "vdjgraph_shard_gather_plan",
@@ -112,6 +117,7 @@ def load_library():
     lib.vdjgraph_fetch.argtypes = [C.c_void_p, C.POINTER(_Result)]
     lib.vdjgraph_stats.argtypes = [C.c_void_p, C.POINTER(_Result)]
     lib.vdjgraph_fetch_pre_table.argtypes = [C.c_void_p, C.POINTER(_PreTable)]
+    lib.vdjgraph_query.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t, C.POINTER(_QueryStats)]
     lib.vdjgraph_host_alloc.argtypes = [C.c_size_t, C.POINTER(C.c_void_p)]
     lib.vdjgraph_host_free.argtypes = [C.c_void_p]
     lib.vdjgraph_host_register.argtypes = [C.c_void_p, C.c_size_t]
@@ -207,6 +213,24 @@ def host_alloc(n_bytes: int) -> np.ndarray:
 
 def host_free(a: np.ndarray):
     load_library().vdjgraph_host_free(C.c_void_p(a.ctypes.data))
+
+
+NIL = 0xFFFFFFFF   # vdjgraph_query's answer for a window with an N or whose k-mer is not a node
+
+
+def query_batch(seqs) -> tuple[np.ndarray, np.ndarray]:
+    """Sequences (bytes or str) -> (text, offsets): one uint8 array of all their bytes and uint64 offsets [n+1];
+    query i is text[offsets[i]:offsets[i+1]], the form vdjgraph_query takes."""
+    bs = [s.encode("latin-1") if isinstance(s, str) else bytes(s) for s in seqs]
+    offsets = np.zeros(len(bs) + 1, np.uint64)
+    np.cumsum(np.fromiter((len(b) for b in bs), np.uint64, count=len(bs)), out=offsets[1:])
+    return np.frombuffer(b"".join(bs), np.uint8), offsets
+
+
+def window_counts(offsets, k: int) -> np.ndarray:
+    """Windows of every query: max(0, len - k + 1)."""
+    lens = np.diff(np.asarray(offsets, np.uint64).astype(np.int64))
+    return np.maximum(lens - (k - 1), 0)
 
 
 @dataclass
@@ -414,6 +438,32 @@ class GraphBuilder:
 
     def shard_release_retired(self):
         self._check(self._lib.vdjgraph_shard_release_retired(self._ctx))
+
+    def query(self, seqs) -> tuple[list[np.ndarray], dict]:
+        """vdjgraph_query: the node (creation rank) of every k-mer window of every sequence in `seqs` (bytes or
+        str over ACGTN), NIL where the window holds an N or its k-mer is not a node of the last built graph.
+        Returns one uint32 view per sequence into a single flat array, and the call's counters."""
+        text, offsets = query_batch(seqs)
+        flat, stats = self.query_flat(text, offsets)
+        ends = np.cumsum(window_counts(offsets, self._p.kmer_size))
+        return (np.split(flat, ends[:-1]) if len(seqs) else []), stats
+
+    def query_flat(self, text, offsets, out: np.ndarray | None = None, n_windows: int | None = None) -> tuple[np.ndarray, dict]:
+        """vdjgraph_query on a batch already in the library's form (query_batch()): the answers of all windows in
+        query order in one uint32 array (`out` when given: one page-locked by vdjgraph_host_alloc or
+        PinnedRecords is written by DMA).  n_windows defaults to the exact count."""
+        t = _as_u8(text)
+        off = np.ascontiguousarray(offsets, np.uint64)
+        if n_windows is None:
+            n_windows = int(window_counts(off, self._p.kmer_size).sum())
+        if out is None:
+            out = np.empty(max(n_windows, 0), np.uint32)
+        if out.dtype != np.uint32 or not out.flags.c_contiguous or out.size < n_windows:
+            raise ValueError("out must be a contiguous uint32 array of at least n_windows elements")
+        st = _QueryStats()
+        self._check(self._lib.vdjgraph_query(self._ctx, t.ctypes.data, off.ctypes.data, max(off.size - 1, 0),
+                                             out.ctypes.data, n_windows, C.byref(st)))
+        return out, {k: (float(getattr(st, k)) if k.startswith("ms_") else int(getattr(st, k))) for k, _ in _QueryStats._fields_}
 
     def pre_table(self) -> PreTable:
         t = _PreTable()
