@@ -42,9 +42,40 @@ typedef enum vdjgraph_status {
     VDJGRAPH_ERR_TOO_MANY_NODES = -4, /* more than MAX_NODES = 900 M distinct gated k-mers (:73, :379) or > 2^32-2 records */
     VDJGRAPH_ERR_CUDA = -5,           /* no device / CUDA runtime error; see vdjgraph_last_error() */
     VDJGRAPH_ERR_NOMEM = -6,
-    VDJGRAPH_ERR_STATE = -7,          /* call sequence violated (e.g. run before stage) */
+    VDJGRAPH_ERR_STATE = -7,          /* call sequence violated (e.g. run before stage); see "Call order" */
     VDJGRAPH_ERR_INTERNAL = -8
 } vdjgraph_status;
+
+/*
+ * Call order.  A context is in one of the states EMPTY, STAGED, COUNTED, PLANNED, PEERS_SET, SCATTERED,
+ * PASSES_DONE, FINISH_PLANNED, FINISH_STEP0, FINISH_STEP1, FINISH_STEP2, FINISHED ("staged": any but EMPTY).
+ * A call made in a state it does not accept fails with VDJGRAPH_ERR_STATE and changes nothing; the message
+ * names the call, the state and the states that accept it.
+ *
+ *   call                              accepted in                              success leaves
+ *   vdjgraph_stage*, _shard_stage*    any                                      STAGED
+ *   vdjgraph_set_params               any                                      EMPTY if read_length or kmer_size
+ *                                                                              changed, else STAGED if staged
+ *   vdjgraph_run                      staged, one rank                         FINISHED
+ *   vdjgraph_shard_count              STAGED, FINISHED                         COUNTED
+ *   vdjgraph_shard_plan               COUNTED                                  PLANNED
+ *   vdjgraph_shard_set_peers          PLANNED .. FINISHED                      PEERS_SET from PLANNED, else unchanged
+ *   vdjgraph_shard_rounds             PLANNED .. FINISHED                      unchanged
+ *   vdjgraph_shard_scatter            PEERS_SET; PASSES_DONE with rounds left  SCATTERED
+ *   vdjgraph_shard_passes             SCATTERED                                PASSES_DONE
+ *   vdjgraph_shard_gather_plan        PASSES_DONE of the last round            FINISH_PLANNED
+ *   vdjgraph_shard_finish_step(s)     FINISH_PLANNED (s = 0), FINISH_STEP<s-1> FINISH_STEP<s>
+ *   vdjgraph_shard_finish             FINISH_STEP2                             FINISHED
+ *   vdjgraph_fetch, _fetch_pre_table  FINISHED, one rank or rank 0             unchanged
+ *   vdjgraph_stats                    FINISHED                                 unchanged
+ *   vdjgraph_query                    FINISHED, one rank                       unchanged
+ *
+ * Calls not listed accept any state.  vdjgraph_fetch_pre_table also needs a one-device, one-round build
+ * (VDJGRAPH_ERR_STATE otherwise).  Any other failure of a staging call leaves EMPTY; of another call on
+ * staged records, STAGED: the records stay staged, and vdjgraph_run or vdjgraph_shard_count builds again.
+ * Failed argument checks (NULL pointers, parameters) and the read-only calls (fetch, stats, pre_table,
+ * query) leave the state as it was.
+ */
 
 /* What the stage reads from the reference's globals, as one POD. */
 typedef struct vdjgraph_params {
@@ -315,8 +346,8 @@ int vdjgraph_fetch_pre_table(vdjgraph_ctx *ctx, vdjgraph_pre_table *out);
  * VDJGRAPH_ERR_PARAM.  On any failure node_of_window is not written.
  *
  * VDJGRAPH_ERR_STATE: no run has finished since the context was created or since the last
- * vdjgraph_stage* / vdjgraph_set_params / vdjgraph_shard_stage*, or the last build ran the sharded
- * phases over more than one rank (each rank's table holds its own share only).
+ * vdjgraph_stage* / vdjgraph_set_params / vdjgraph_shard_stage* or a failed call, or the last build ran
+ * the sharded phases over more than one rank (each rank's table holds its own share only).
  * Synchronous, on the context's stream; the graph and what vdjgraph_fetch returns are unchanged.
  */
 typedef struct vdjgraph_query_stats {

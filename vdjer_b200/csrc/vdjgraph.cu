@@ -206,10 +206,9 @@ static_assert(EV_FINISH_END == EV_FINISH + 7, "the finish's events are consecuti
 
 /* The finished graph's survivor table as vdjgraph_query looks k-mers up in it: the table k_export read
  * (one round: d_t2 with the per-unit slices of the plan; several rounds: the merged flat table d_t2m)
- * and the slicing and geometry it was read with.  Valid from the end of a one-device finish until the
- * next stage, set_params or run; table is null when the graph has no nodes. */
+ * and the slicing and geometry it was read with.  Recorded by a one-device finish, current while the context
+ * is queryable(); table is null when the graph has no nodes. */
 struct GraphView {
-    bool valid = false;
     const Slot2 *table = nullptr;
     uint64_t cap = 0, n_nodes = 0;
     Part pt{};
@@ -256,9 +255,10 @@ constexpr uint64_t SLICE_BYTES = 12ull << 20;   /* table-1 bytes one hash unit a
 enum { BUF_BASES = 0, BUF_VALID, BUF_QUAL, BUF_STRAND, BUF_TUPLES, BUF_GATHER, NBUF };
 static_assert(NBUF == VDJGRAPH_SHARD_NBUF, "header and library disagree");
 
-/* where a build stands: what has happened last.  FINISH_STEPn: step n of the finish has been queued or done
- * (the three are consecutive, see finish_step_phase). */
-enum class Phase { STAGED, COUNTED, PLANNED, SCATTERED, PASSES_DONE, FINISH_PLANNED, FINISH_STEP0, FINISH_STEP1, FINISH_STEP2, FINISHED };
+/* What a context may do next (include/vdjgraph.h, "Call order"): the last step of staging or of a build it has completed.
+ * FINISH_STEPn: step n of the finish has been queued or done; FINISH_PLANNED and the three steps are consecutive. */
+enum class State { EMPTY, STAGED, COUNTED, PLANNED, PEERS_SET, SCATTERED, PASSES_DONE, FINISH_PLANNED, FINISH_STEP0, FINISH_STEP1,
+                   FINISH_STEP2, FINISHED };
 
 struct Shard {
     int G = 1, rank = 0;
@@ -274,7 +274,6 @@ struct Shard {
     double slot_scale = 1.0;                      /* table-1 slots per estimated k-mer, relative to the default */
     bool ignore_hint = false;                     /* the caller's table_capacity turned out too small */
     void *peer[MAX_DEV][NBUF] = {};
-    bool peers_set = false;
     uint64_t n_runs_own = 0, n_gated_own = 0;     /* what this device receives in the current round */
     uint64_t n_gated_src = 0, n_valid_src = 0;    /* windows this device produces */
     double est_distinct = 0;
@@ -285,7 +284,6 @@ struct Shard {
     float acc[6] = {};                            /* scatter, init1, pass1, prune, table2, pass2 ms summed over the rounds */
     bool merged() const { return G > 1 || S > 1; } /* the finish builds a table over survivor RECORDS */
     uint64_t bar_seq = 0;                         /* device barriers of this build so far (k_peer_barrier) */
-    Phase phase = Phase::STAGED;
 };
 
 struct vdjgraph_ctx {
@@ -296,7 +294,7 @@ struct vdjgraph_ctx {
     Geom g;
     uint64_t R_pad = 0;
     bool any_strand1 = false;
-    bool staged = false, ran = false, staged_direct = false;
+    State state = State::EMPTY;   /* here, not in Shard: staging resets Shard */
     cudaStream_t stream = nullptr;
     cudaEvent_t ev[EV_COUNT] = {};
     std::vector<StageWorker> workers;
@@ -330,6 +328,11 @@ struct vdjgraph_ctx {
 
     GraphView view;   /* what vdjgraph_query looks k-mers up in */
     QueryBufs q;
+
+    /* what a finished build leaves: the graph (on rank 0 of a sharded build) and a table that holds all of it (one rank) */
+    bool has_graph() const { return state == State::FINISHED && (sh.G == 1 || sh.rank == 0); }
+    bool queryable() const { return state == State::FINISHED && sh.G == 1; }
+    bool rounds_left() const { return sh.rnd + 1 < sh.S; }
 };
 
 namespace {
@@ -624,8 +627,8 @@ extern "C" int vdjgraph_set_params(vdjgraph_ctx *c, const vdjgraph_params *param
     int dev = c->prm.device;
     c->prm = *params;
     c->prm.device = dev;
-    if (regeom) { c->staged = false; }
-    c->ran = false; c->view.valid = false;
+    /* the build is dropped; the staged records stay unless their geometry changed */
+    c->state = regeom ? State::EMPTY : std::min(c->state, State::STAGED);
     return 0;
 }
 
@@ -633,14 +636,26 @@ namespace { int count_begin(vdjgraph_ctx *c); int count_end(vdjgraph_ctx *c); }
 
 /* np / ns count TEXT records.  fwd = 0: the reference's buffers (every read followed by its reverse
  * complement).  fwd = 1: forward reads only; the packed read set is the same as if the reverse
- * complements had been in the text (packed record 2i = read i, 2i+1 = derived by k_pack). */
-static int stage_impl(vdjgraph_ctx *c, const char *primary, size_t np, const char *secondary, size_t ns, uint32_t fwd) {
+ * complements had been in the text (packed record 2i = read i, 2i+1 = derived by k_pack).
+ * info: this rank's share of a sharded build (vdjgraph_shard_stage*), NULL for one device. */
+static int stage_impl(vdjgraph_ctx *c, const char *primary, size_t np, const char *secondary, size_t ns, uint32_t fwd,
+                      const vdjgraph_shard_info *info) {
     if (!c) return fail(VDJGRAPH_ERR_PARAM, "ctx is NULL");
     if ((np && !primary) || (ns && !secondary)) return fail(VDJGRAPH_ERR_PARAM, "NULL record buffer");
-    CK(cudaSetDevice(c->device));
-    c->staged = false; c->ran = false; c->view.valid = false;
+    c->state = State::EMPTY;   /* until the records are staged */
     const uint64_t Rt = (uint64_t)np + (uint64_t)ns;   /* text records */
     const uint64_t R = Rt << fwd;                      /* packed records */
+    if (info) {
+        const uint32_t G = info->n_ranks;
+        if (G < 1 || G > (uint32_t)MAX_DEV || (G & (G - 1)) || info->rank >= G)
+            return fail(VDJGRAPH_ERR_PARAM, "n_ranks %u must be 1, 2, 4 or 8 and rank %u below it", G, info->rank);
+        if (info->record_base + R > info->total_records)
+            return fail(VDJGRAPH_ERR_PARAM, "record range exceeds total_records");
+        if (info->total_records > 0xFFFFFFFEull)
+            return fail(VDJGRAPH_ERR_TOO_MANY_NODES, "%llu records exceed the 2^32-2 record limit", (unsigned long long)info->total_records);
+        for (DevBuf *b : c->peer_bufs()) b->exported = G > 1;
+    }
+    CK(cudaSetDevice(c->device));
     if (R > 0xFFFFFFFEull) return fail(VDJGRAPH_ERR_TOO_MANY_NODES, "%llu records exceed the 2^32-2 record limit", (unsigned long long)R);
     double t0 = wall_ms();
     make_geom(c, R);
@@ -671,7 +686,6 @@ static int stage_impl(vdjgraph_ctx *c, const char *primary, size_t np, const cha
         CK(cudaStreamSynchronize(c->stream));   /* padding memsets, flags and zeroed counters are in place before the workers start */
         const bool direct = is_page_locked(primary, np * rec_len) && is_page_locked(secondary, ns * rec_len);
         if ((rc = direct ? stage_direct(c, primary, np, secondary, Rt, fwd) : stage_pageable(c, primary, np, secondary, Rt, fwd))) return rc;
-        c->staged_direct = direct;
         CK(cudaMemcpyAsync(hb, c->d_bad.p, 3 * sizeof(uint64_t), cudaMemcpyDeviceToHost, c->stream));
         CK(cudaStreamSynchronize(c->stream));
         if (hb[0] != ~0ull)
@@ -691,17 +705,20 @@ static int stage_impl(vdjgraph_ctx *c, const char *primary, size_t np, const cha
     c->res.n_records = R;
     c->res.n_windows = R * (uint64_t)g.w;
     c->sh = Shard();
-    c->sh.total_records = R;
-    c->sh.rec_base[1] = R;
-    c->staged = true;
+    Shard &sh = c->sh;
+    if (info) { sh.G = (int)info->n_ranks; sh.rank = (int)info->rank; }
+    sh.total_records = info ? info->total_records : R;
+    sh.rec_base[sh.rank] = info ? info->record_base : 0;   /* the other ranks' arrive with vdjgraph_shard_plan */
+    sh.rec_base[sh.rank + 1] = sh.rec_base[sh.rank] + R;
+    c->state = State::STAGED;
     return 0;
 }
 
 extern "C" int vdjgraph_stage(vdjgraph_ctx *c, const char *primary, size_t np, const char *secondary, size_t ns) {
-    return stage_impl(c, primary, np, secondary, ns, 0);
+    return stage_impl(c, primary, np, secondary, ns, 0, nullptr);
 }
 extern "C" int vdjgraph_stage_forward(vdjgraph_ctx *c, const char *primary_reads, size_t np, const char *secondary_reads, size_t ns) {
-    return stage_impl(c, primary_reads, np, secondary_reads, ns, 1);
+    return stage_impl(c, primary_reads, np, secondary_reads, ns, 1, nullptr);
 }
 
 /* ========================================================================================== */
@@ -713,16 +730,24 @@ extern "C" int vdjgraph_stage_forward(vdjgraph_ctx *c, const char *primary_reads
 /* ========================================================================================== */
 namespace {
 
+const char *const STATE_NAMES[] = { "EMPTY", "STAGED", "COUNTED", "PLANNED", "PEERS_SET", "SCATTERED", "PASSES_DONE",
+                                    "FINISH_PLANNED", "FINISH_STEP0", "FINISH_STEP1", "FINISH_STEP2", "FINISHED" };
+static_assert(sizeof(STATE_NAMES) / sizeof(*STATE_NAMES) == (size_t)State::FINISHED + 1, "a name per state");
 
-int phase_check(vdjgraph_ctx *c, Phase want, const char *what) {
+/* sets of states: bit(s), and from(s) = s .. FINISHED */
+constexpr unsigned bit(State s) { return 1u << (int)s; }
+constexpr unsigned from(State s) { return 2 * bit(State::FINISHED) - bit(s); }
+
+/* The check of call order: `call` is accepted when the context is in a state of `accepted` and the caller gives no `refusal`
+ * (a reason the sequence rules it out in that state).  A refused call fails with VDJGRAPH_ERR_STATE and changes nothing. */
+int check_state(const vdjgraph_ctx *c, const char *call, unsigned accepted, const char *refusal = nullptr) {
     if (!c) return fail(VDJGRAPH_ERR_PARAM, "ctx is NULL");
-    if (!c->staged) return fail(VDJGRAPH_ERR_STATE, "%s before vdjgraph_stage", what);
-    if (c->sh.phase != want) return fail(VDJGRAPH_ERR_STATE, "%s called in phase %d (expected %d)", what, (int)c->sh.phase, (int)want);
-    return 0;
+    if (accepted & bit(c->state)) return refusal ? fail(VDJGRAPH_ERR_STATE, "%s", refusal) : 0;
+    std::string names;
+    for (int s = 0; s <= (int)State::FINISHED; s++)
+        if (accepted & bit(State(s))) { names += names.empty() ? "" : ", "; names += STATE_NAMES[s]; }
+    return fail(VDJGRAPH_ERR_STATE, "%s in state %s; it is accepted in %s", call, STATE_NAMES[(int)c->state], names.c_str());
 }
-
-/* the phase once finish step `step` (0, 1, 2) has been queued */
-Phase finish_step_phase(int step) { return Phase((int)Phase::FINISH_STEP0 + step); }
 
 /* the device counters to the host (c->h_ctr), the stream synchronised */
 int read_counters(vdjgraph_ctx *c) {
@@ -994,8 +1019,6 @@ int run_plan(vdjgraph_ctx *c, const uint64_t *hist_all, const uint8_t *hll) {
     c->res.n_runs = 0;
     for (int u = 0; u < sh.NU; u++) c->res.n_runs += sh.runs[(size_t)sh.rank * sh.NU + u];
     c->res.run_bytes = (uint32_t)(RUN_WORDS * 8);
-    sh.peers_set = false;
-    sh.phase = Phase::PLANNED;
     return 0;
 }
 
@@ -1004,15 +1027,9 @@ void own_buffers(vdjgraph_ctx *c, void **ptrs, size_t *bytes) {
     for (int i = 0; i < NBUF; i++) { ptrs[i] = b[i]->p; if (bytes) bytes[i] = b[i]->cap; }
 }
 
-void set_self_peers(vdjgraph_ctx *c) {
-    own_buffers(c, c->sh.peer[c->sh.rank], nullptr);
-    c->sh.peers_set = true;
-}
-
 /* K1: scatter this device's runs into the buffers of the units' owners */
 int run_scatter(vdjgraph_ctx *c) {
     Shard &sh = c->sh;
-    if (!sh.peers_set) return fail(VDJGRAPH_ERR_STATE, "peer buffers not set");
     const Geom g = c->g;
     cudaStream_t s = c->stream;
     const int G = sh.G, NU = sh.NU;
@@ -1066,7 +1083,6 @@ int run_scatter(vdjgraph_ctx *c) {
     }
     CK(cudaEventRecord(c->ev[EV_SCATTER_END], s));
     if (G > 1) CK(cudaStreamSynchronize(s));   /* the peers' runs are complete once every device got here */
-    sh.phase = Phase::SCATTERED;
     return 0;
 }
 
@@ -1243,7 +1259,6 @@ int run_passes(vdjgraph_ctx *c) {
         sh.surv_done = n_surv;
     }
     sh.surv_all[sh.rank] = sh.surv_done;
-    sh.phase = Phase::PASSES_DONE;
     return 0;
 }
 
@@ -1382,11 +1397,8 @@ int run_finish(vdjgraph_ctx *c) {
     }
     take_times(c);
     cudaEventElapsedTime(&res.ms_device, c->ev[EV_BUILD], c->ev[EV_FINISH_END]);
-    sh.phase = Phase::FINISHED;
-    c->ran = true;
     c->view.table = n_surv ? table : nullptr;
     c->view.cap = cap2; c->view.n_nodes = n_surv; c->view.pt = pt; c->view.g = g;
-    c->view.valid = true;
     return 0;
 }
 
@@ -1523,7 +1535,6 @@ int finish_step(vdjgraph_ctx *c, int step, bool device_barrier) {
         CK(cudaStreamSynchronize(s));
     }
     CK(cudaEventRecord(c->ev[EV_STEP0_MET + 2 * step], s));
-    sh.phase = finish_step_phase(step);
     return 0;
 }
 
@@ -1576,8 +1587,6 @@ int finish_end(vdjgraph_ctx *c) {
     res.ms_device = res.ms_scatter + res.ms_init1 + res.ms_pass1 + res.ms_prune + res.ms_table2 + res.ms_pass2 + res.ms_export;
     res.n_nodes = sh.rank == 0 ? f.n_total : 0;
     if (sh.rank == 0) res.n_pre = f.n_total;   /* (the other ranks keep their own survivor count) */
-    sh.phase = Phase::FINISHED;
-    c->ran = sh.rank == 0;
     return 0;
 }
 
@@ -1585,83 +1594,61 @@ int finish_end(vdjgraph_ctx *c) {
 
 extern "C" int vdjgraph_run(vdjgraph_ctx *c) {
     if (!c) return fail(VDJGRAPH_ERR_PARAM, "ctx is NULL");
-    if (!c->staged) return fail(VDJGRAPH_ERR_STATE, "vdjgraph_run before vdjgraph_stage");
-    if (c->sh.G != 1) return fail(VDJGRAPH_ERR_STATE, "vdjgraph_run on a sharded context; use the vdjgraph_shard_* phases");
+    int rc = check_state(c, "vdjgraph_run", from(State::STAGED),
+                         c->sh.G == 1 ? nullptr : "vdjgraph_run on a sharded context; use the vdjgraph_shard_* phases");
+    if (rc) return rc;
+    c->state = State::STAGED;   /* until the build has finished */
     CK(cudaSetDevice(c->device));
-    c->ran = false; c->view.valid = false;
-    int rc;
     if (c->g.R == 0) {
         reset_run_stats(c);
-        c->ran = true;
         c->view = GraphView();   /* no nodes: every window answers NIL */
-        c->view.g = c->g; c->view.valid = true;
-        return 0;
+        c->view.g = c->g;
+    } else {
+        if ((rc = run_plan(c, c->h_hist.as<uint64_t>(), c->h_hll.as<uint8_t>()))) return rc;
+        own_buffers(c, c->sh.peer[c->sh.rank], nullptr);   /* the only peer */
+        for (int r = 0; r < c->sh.S; r++) {
+            c->sh.rnd = r;
+            if ((rc = run_scatter(c))) return rc;
+            if ((rc = run_passes(c))) return rc;
+        }
+        if ((rc = run_finish(c))) return rc;
     }
-    if ((rc = run_plan(c, c->h_hist.as<uint64_t>(), c->h_hll.as<uint8_t>()))) return rc;
-    set_self_peers(c);
-    for (int r = 0; r < c->sh.S; r++) {
-        c->sh.rnd = r;
-        if ((rc = run_scatter(c))) return rc;
-        if ((rc = run_passes(c))) return rc;
-    }
-    return run_finish(c);
+    c->state = State::FINISHED;
+    return 0;
 }
 
 /* ---------------------------------------------------------------------------------------- */
 /* sharded build: the same phases, driven by the caller                                       */
 /* ---------------------------------------------------------------------------------------- */
-static int shard_stage_impl(vdjgraph_ctx *c, const char *primary, size_t np, const char *secondary, size_t ns,
-                            const vdjgraph_shard_info *info, uint32_t fwd) {
-    if (!c || !info) return fail(VDJGRAPH_ERR_PARAM, "NULL argument");
-    const uint32_t G = info->n_ranks;
-    if (G < 1 || G > (uint32_t)MAX_DEV || (G & (G - 1)) || info->rank >= G)
-        return fail(VDJGRAPH_ERR_PARAM, "n_ranks %u must be 1, 2, 4 or 8 and rank %u below it", G, info->rank);
-    const uint64_t n_rec = ((uint64_t)np + (uint64_t)ns) << fwd;   /* packed records of this rank */
-    if (info->record_base + n_rec > info->total_records)
-        return fail(VDJGRAPH_ERR_PARAM, "record range exceeds total_records");
-    if (info->total_records > 0xFFFFFFFEull)
-        return fail(VDJGRAPH_ERR_TOO_MANY_NODES, "%llu records exceed the 2^32-2 record limit", (unsigned long long)info->total_records);
-    for (DevBuf *b : c->peer_bufs()) b->exported = G > 1;
-    int rc = stage_impl(c, primary, np, secondary, ns, fwd);
-    if (rc) return rc;
-    Shard &sh = c->sh;
-    sh.G = (int)G; sh.rank = (int)info->rank;
-    sh.total_records = info->total_records;
-    memset(sh.rec_base, 0, sizeof(sh.rec_base));
-    sh.rec_base[sh.rank] = info->record_base;   /* the others arrive with vdjgraph_shard_plan */
-    sh.rec_base[sh.rank + 1] = info->record_base + n_rec;
-    return 0;
-}
-
 extern "C" int vdjgraph_shard_stage(vdjgraph_ctx *c, const char *primary, size_t np, const char *secondary, size_t ns,
                                     const vdjgraph_shard_info *info) {
-    return shard_stage_impl(c, primary, np, secondary, ns, info, 0);
+    return info ? stage_impl(c, primary, np, secondary, ns, 0, info) : fail(VDJGRAPH_ERR_PARAM, "NULL argument");
 }
 /* forward reads only (vdjgraph_stage_forward); record_base / total_records / the record counts handed
  * to vdjgraph_shard_plan stay in the doubled numbering (two records per read) */
 extern "C" int vdjgraph_shard_stage_forward(vdjgraph_ctx *c, const char *primary_reads, size_t np, const char *secondary_reads,
                                             size_t ns, const vdjgraph_shard_info *info) {
-    return shard_stage_impl(c, primary_reads, np, secondary_reads, ns, info, 1);
+    return info ? stage_impl(c, primary_reads, np, secondary_reads, ns, 1, info) : fail(VDJGRAPH_ERR_PARAM, "NULL argument");
 }
 
-/* the per-bucket counts and HyperLogLog registers of this rank's staged records (k_count ran with the staging) */
+/* the per-bucket counts and HyperLogLog registers of this rank's staged records (k_count ran with the staging);
+ * after a finished build, the next build of the same records */
 extern "C" int vdjgraph_shard_count(vdjgraph_ctx *c, uint64_t *hist, uint8_t *hll) {
-    if (c && c->staged && c->sh.phase == Phase::FINISHED) c->sh.phase = Phase::STAGED;   /* another build of the same staged records */
-    int rc = phase_check(c, Phase::STAGED, "vdjgraph_shard_count");
+    int rc = check_state(c, "vdjgraph_shard_count", bit(State::STAGED) | bit(State::FINISHED));
     if (rc) return rc;
     if (!hist || !hll) return fail(VDJGRAPH_ERR_PARAM, "NULL argument");
-    c->ran = false; c->view.valid = false;
     memcpy(hist, c->h_hist.p, HIST_WORDS * sizeof(uint64_t));
     memcpy(hll, c->h_hll.p, HLL_BYTES);
-    c->sh.phase = Phase::COUNTED;
+    c->state = State::COUNTED;
     return 0;
 }
 
 extern "C" int vdjgraph_shard_plan(vdjgraph_ctx *c, const uint64_t *hist_all, const uint8_t *hll_merged,
                                    const uint64_t *record_counts) {
-    int rc = phase_check(c, Phase::COUNTED, "vdjgraph_shard_plan");
+    int rc = check_state(c, "vdjgraph_shard_plan", bit(State::COUNTED));
     if (rc) return rc;
     if (!hist_all || !hll_merged || !record_counts) return fail(VDJGRAPH_ERR_PARAM, "NULL argument");
+    c->state = State::STAGED;   /* until the plan is made */
     CK(cudaSetDevice(c->device));
     Shard &sh = c->sh;
     uint64_t base = 0;
@@ -1674,6 +1661,7 @@ extern "C" int vdjgraph_shard_plan(vdjgraph_ctx *c, const uint64_t *hist_all, co
      * several host exchanges; those of the last build arrived before its final one) */
     sh.bar_seq = 0;
     if (sh.G > 1 && c->d_gather.p) CK(cudaMemset(c->d_gather.p, 0, FLAGS_BYTES));
+    c->state = State::PLANNED;
     return 0;
 }
 
@@ -1685,45 +1673,52 @@ extern "C" int vdjgraph_shard_buffers(vdjgraph_ctx *c, void **ptrs, size_t *byte
 
 extern "C" int vdjgraph_shard_set_peers(vdjgraph_ctx *c, void *const *ptrs) {
     if (!c || !ptrs) return fail(VDJGRAPH_ERR_PARAM, "NULL argument");
-    if (c->sh.phase < Phase::PLANNED) return fail(VDJGRAPH_ERR_STATE, "vdjgraph_shard_set_peers before vdjgraph_shard_plan");
+    int rc = check_state(c, "vdjgraph_shard_set_peers", from(State::PLANNED));
+    if (rc) return rc;
     Shard &sh = c->sh;
     for (int d = 0; d < sh.G; d++)
         for (int i = 0; i < NBUF; i++) sh.peer[d][i] = ptrs[d * NBUF + i];
-    set_self_peers(c);
+    own_buffers(c, sh.peer[sh.rank], nullptr);
+    if (c->state == State::PLANNED) c->state = State::PEERS_SET;   /* called again for the finish: the state stays */
     return 0;
 }
 
 extern "C" int vdjgraph_shard_rounds(vdjgraph_ctx *c) {
-    if (!c) return fail(VDJGRAPH_ERR_PARAM, "ctx is NULL");
-    if (!c->staged || c->sh.phase < Phase::PLANNED) return fail(VDJGRAPH_ERR_STATE, "vdjgraph_shard_rounds before vdjgraph_shard_plan");
-    return c->sh.S;
+    int rc = check_state(c, "vdjgraph_shard_rounds", from(State::PLANNED));
+    return rc ? rc : c->sh.S;
 }
 
 extern "C" int vdjgraph_shard_scatter(vdjgraph_ctx *c) {
-    /* after the passes of a round that was not the last: the next round */
-    if (c && c->staged && c->sh.phase == Phase::PASSES_DONE && c->sh.rnd + 1 < c->sh.S) { c->sh.rnd++; c->sh.phase = Phase::PLANNED; }
-    int rc = phase_check(c, Phase::PLANNED, "vdjgraph_shard_scatter");
+    if (!c) return fail(VDJGRAPH_ERR_PARAM, "ctx is NULL");
+    /* the first round once the peers are set, each further one after the passes of the round before */
+    int rc = check_state(c, "vdjgraph_shard_scatter", bit(State::PEERS_SET) | (c->rounds_left() ? bit(State::PASSES_DONE) : 0));
     if (rc) return rc;
+    if (c->state == State::PASSES_DONE) c->sh.rnd++;
+    c->state = State::STAGED;   /* until the runs are scattered */
     CK(cudaSetDevice(c->device));
-    return run_scatter(c);
+    if ((rc = run_scatter(c))) return rc;
+    c->state = State::SCATTERED;
+    return 0;
 }
 
 extern "C" int vdjgraph_shard_passes(vdjgraph_ctx *c, uint64_t *n_survivors) {
-    int rc = phase_check(c, Phase::SCATTERED, "vdjgraph_shard_passes");
+    int rc = check_state(c, "vdjgraph_shard_passes", bit(State::SCATTERED));
     if (rc) return rc;
+    c->state = State::STAGED;   /* until the passes are done */
     CK(cudaSetDevice(c->device));
     if ((rc = run_passes(c))) return rc;
     if (c->sh.G == 1) { CK(cudaStreamSynchronize(c->stream)); }
     if (n_survivors) *n_survivors = c->sh.surv_all[c->sh.rank];
+    c->state = State::PASSES_DONE;
     return 0;
 }
 
 extern "C" int vdjgraph_shard_gather_plan(vdjgraph_ctx *c, const uint64_t *survivors_all) {
-    int rc = phase_check(c, Phase::PASSES_DONE, "vdjgraph_shard_gather_plan");
+    if (!c || !survivors_all) return fail(VDJGRAPH_ERR_PARAM, "NULL argument");
+    int rc = check_state(c, "vdjgraph_shard_gather_plan", bit(State::PASSES_DONE),
+                         c->rounds_left() ? "vdjgraph_shard_gather_plan before the last round: vdjgraph_shard_scatter comes next" : nullptr);
     if (rc) return rc;
-    if (!survivors_all) return fail(VDJGRAPH_ERR_PARAM, "NULL argument");
-    if (c->sh.rnd + 1 < c->sh.S)
-        return fail(VDJGRAPH_ERR_STATE, "vdjgraph_shard_gather_plan after round %d of %d", c->sh.rnd + 1, c->sh.S);
+    c->state = State::STAGED;   /* until the finish is planned */
     CK(cudaSetDevice(c->device));
     Shard &sh = c->sh;
     if (survivors_all[sh.rank] != sh.surv_done)
@@ -1732,7 +1727,7 @@ extern "C" int vdjgraph_shard_gather_plan(vdjgraph_ctx *c, const uint64_t *survi
     for (int d = 0; d < sh.G; d++) { sh.surv_all[d] = survivors_all[d]; sh.surv_off[d] = off; off += survivors_all[d]; }
     sh.surv_off[sh.G] = off;
     if (sh.G > 1 && (rc = finish_plan(c))) return rc;
-    sh.phase = Phase::FINISH_PLANNED;
+    c->state = State::FINISH_PLANNED;
     return 0;
 }
 
@@ -1744,18 +1739,25 @@ extern "C" int vdjgraph_shard_finish_bytes(vdjgraph_ctx *c, const uint64_t *surv
 
 extern "C" int vdjgraph_shard_finish_step(vdjgraph_ctx *c, int step, int device_barrier) {
     if (step < 0 || step > 2) return fail(VDJGRAPH_ERR_PARAM, "finish step %d", step);
-    int rc = phase_check(c, step ? finish_step_phase(step - 1) : Phase::FINISH_PLANNED, "vdjgraph_shard_finish_step");
+    const State before = State((int)State::FINISH_PLANNED + step);   /* FINISH_PLANNED or the step before */
+    int rc = check_state(c, "vdjgraph_shard_finish_step", bit(before));
     if (rc) return rc;
+    c->state = State::STAGED;   /* until the step is queued */
     CK(cudaSetDevice(c->device));
-    if (c->sh.G == 1) { c->sh.phase = finish_step_phase(step); return 0; }   /* one device: everything happens in vdjgraph_shard_finish */
-    return finish_step(c, step, device_barrier != 0);
+    /* one device: everything happens in vdjgraph_shard_finish */
+    if (c->sh.G > 1 && (rc = finish_step(c, step, device_barrier != 0))) return rc;
+    c->state = State((int)before + 1);
+    return 0;
 }
 
 extern "C" int vdjgraph_shard_finish(vdjgraph_ctx *c) {
-    int rc = phase_check(c, Phase::FINISH_STEP2, "vdjgraph_shard_finish");
+    int rc = check_state(c, "vdjgraph_shard_finish", bit(State::FINISH_STEP2));
     if (rc) return rc;
+    c->state = State::STAGED;   /* until the graph is finished */
     CK(cudaSetDevice(c->device));
-    return c->sh.G == 1 ? run_finish(c) : finish_end(c);
+    if ((rc = c->sh.G == 1 ? run_finish(c) : finish_end(c))) return rc;
+    c->state = State::FINISHED;
+    return 0;
 }
 
 /* Frees allocations that were replaced by larger ones while peers could still have them mapped.
@@ -1829,12 +1831,12 @@ extern "C" int vdjgraph_host_unregister(void *p) {
 
 extern "C" int vdjgraph_fetch(vdjgraph_ctx *c, vdjgraph_result *out) {
     if (!c || !out) return fail(VDJGRAPH_ERR_PARAM, "NULL argument");
-    if (!c->ran) return fail(VDJGRAPH_ERR_STATE, "vdjgraph_fetch before vdjgraph_run");
+    int rc = check_state(c, "vdjgraph_fetch", bit(State::FINISHED), c->has_graph() ? nullptr : "vdjgraph_fetch on a rank other than 0");
+    if (rc) return rc;
     CK(cudaSetDevice(c->device));
     double t0 = wall_ms();
     vdjgraph_result &r = c->res;
     uint64_t bytes = 0;
-    int rc;
     if ((rc = c->nodes.fetch(r.n_nodes, c->prm.flags & VDJGRAPH_FLAG_EXPORT_KEYS, c->stream, r, bytes))) return rc;
     if (c->res.hm_buckets) {   /* the layout exists even for an empty graph: 32 empty buckets */
         cudaStream_t s = c->stream;
@@ -1852,7 +1854,7 @@ extern "C" int vdjgraph_fetch(vdjgraph_ctx *c, vdjgraph_result *out) {
 
 extern "C" int vdjgraph_stats(vdjgraph_ctx *c, vdjgraph_result *out) {
     if (!c || !out) return fail(VDJGRAPH_ERR_PARAM, "NULL argument");
-    if (!c->ran && c->sh.phase < Phase::FINISHED) return fail(VDJGRAPH_ERR_STATE, "vdjgraph_stats before vdjgraph_run");
+    if (int rc = check_state(c, "vdjgraph_stats", bit(State::FINISHED))) return rc;
     *out = c->res;
     out->first_pos = nullptr; out->frequency = nullptr; out->out_deg = out->in_deg = nullptr;
     out->out_succ = out->in_pred = nullptr; out->kmer_lo = out->kmer_hi = nullptr; out->hm_slots = nullptr;
@@ -1877,12 +1879,13 @@ extern "C" int vdjgraph_build_forward(vdjgraph_ctx *c, const char *primary_reads
 
 extern "C" int vdjgraph_fetch_pre_table(vdjgraph_ctx *c, vdjgraph_pre_table *out) {
     if (!c || !out) return fail(VDJGRAPH_ERR_PARAM, "NULL argument");
-    if (!c->ran) return fail(VDJGRAPH_ERR_STATE, "vdjgraph_fetch_pre_table before vdjgraph_run");
+    int rc = check_state(c, "vdjgraph_fetch_pre_table", bit(State::FINISHED),
+                         c->has_graph() ? nullptr : "vdjgraph_fetch_pre_table on a rank other than 0");
+    if (rc) return rc;
     if (c->sh.merged()) return fail(VDJGRAPH_ERR_STATE, "the pruned pass-1 table is only kept by a one-device, one-round build");
     CK(cudaSetDevice(c->device));
     const uint64_t n = c->res.n_pre;
     const size_t na = std::max<uint64_t>(n, 1);
-    int rc;
     if ((rc = c->d_pre_klo.ensure(na * 8)) || (rc = c->d_pre_khi.ensure(na * 8)) || (rc = c->d_pre_freq.ensure(na * 2)) ||
         (rc = c->d_pre_n.ensure(8)) || (rc = c->h_pre_klo.ensure(na * 8)) || (rc = c->h_pre_khi.ensure(na * 8)) ||
         (rc = c->h_pre_freq.ensure(na * 2)) || (rc = c->h_pre_n.ensure(8)))
@@ -1913,12 +1916,10 @@ extern "C" int vdjgraph_fetch_pre_table(vdjgraph_ctx *c, vdjgraph_pre_table *out
 extern "C" int vdjgraph_query(vdjgraph_ctx *c, const char *seqs, const uint64_t *offsets, size_t nq,
                               uint32_t *out, size_t n_windows, vdjgraph_query_stats *stats) {
     const double t0 = wall_ms();
-    if (!c) return fail(VDJGRAPH_ERR_PARAM, "ctx is NULL");
-    if (!c->view.valid) {
-        if (c->sh.G > 1 && c->sh.phase == Phase::FINISHED)
-            return fail(VDJGRAPH_ERR_STATE, "vdjgraph_query on a graph built over %d ranks: each rank's table holds its own share", c->sh.G);
-        return fail(VDJGRAPH_ERR_STATE, "vdjgraph_query before vdjgraph_run (or after vdjgraph_stage / vdjgraph_set_params)");
-    }
+    int rc = check_state(c, "vdjgraph_query", bit(State::FINISHED));
+    if (rc) return rc;
+    if (!c->queryable())
+        return fail(VDJGRAPH_ERR_STATE, "vdjgraph_query on a graph built over %d ranks: each rank's table holds its own share", c->sh.G);
     if (nq && !offsets) return fail(VDJGRAPH_ERR_PARAM, "offsets is NULL");
     const GraphView &v = c->view;
     const uint64_t k = (uint64_t)v.g.k;
@@ -1935,7 +1936,6 @@ extern "C" int vdjgraph_query(vdjgraph_ctx *c, const char *seqs, const uint64_t 
     CK(cudaSetDevice(c->device));
     cudaStream_t s = c->stream;
     QueryBufs &qb = c->q;
-    int rc;
     if ((rc = qb.init())) return rc;
     const double chunk_kb = env_double("VDJGRAPH_QUERY_CHUNK_KB", 0);
     const uint64_t CH = chunk_kb > 0 ? std::max<uint64_t>(64, (uint64_t)(chunk_kb * 1024)) : QUERY_CHUNK;
