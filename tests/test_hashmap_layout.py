@@ -62,3 +62,17 @@ def test_layout_of_sharded_and_multi_round_builds(built):
     with GraphBuilder(L, k, mf, mq, hashmap_layout=True, rounds=4) as gb:
         got = gb.build(primary, secondary)
     assert np.array_equal(got.hm_slots, want)
+    from vdjer_b200 import MultiBuilder, shard
+    for G in (2, 4):
+        total = (primary.size // (2 * L + 1)) + (secondary.size // (2 * L + 1))
+        parts = [shard.split_records(primary, secondary, L, lo, hi) for lo, hi in shard.shard_ranges(total, G)]
+        builders = [GraphBuilder(L, k, mf, mq, device=0, hashmap_layout=True, rounds=2 if G == 2 else 0) for _ in range(G)]
+        try:
+            got = shard.build_local(builders, parts)
+        finally:
+            for b in builders:
+                b.close()
+        assert got.stats["hm_buckets"] == nb and np.array_equal(got.hm_slots, want), f"sharded G={G}"
+    with MultiBuilder(L, k, mf, mq, devices=[0, 0], hashmap_layout=True) as mb:
+        got = mb.build(primary, secondary)
+    assert got.stats["hm_buckets"] == nb and np.array_equal(got.hm_slots, want), "multi"

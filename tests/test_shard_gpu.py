@@ -5,12 +5,15 @@ across processes the same phases run over CUDA IPC mappings, see vdjer_b200/shar
 tests/test_shard_dist.py): every tuple is written by the scatter kernel into the buffer of the
 rank that owns its hash partition, reads are compared and quality rows fetched across ranks, and
 rank 0 finishes over the gathered survivor records."""
+import os
+
 import numpy as np
 import pytest
 
 from oracle import loader
-from tests.util import assert_graph_equal
-from vdjer_b200 import GraphBuilder, shard, synth
+from tests.cases import CASES, make_inputs
+from tests.util import GOLDEN_DIR, assert_graph_equal
+from vdjer_b200 import GraphBuilder, MultiBuilder, shard, synth
 
 pytestmark = pytest.mark.gpu
 
@@ -122,3 +125,67 @@ def test_sharded_from_forward_reads_only(built, G):
         for b in builders:
             b.close()
     assert_graph_equal(got, want, f"forward G={G}")
+
+
+def _exports_equal(got, single, what):
+    """The k-mer array and the hash-map layout of a sharded finish equal the one-device build's."""
+    for name in ["kmer_lo", "kmer_hi", "hm_slots"]:
+        a, b = getattr(got, name), getattr(single, name)
+        assert a is not None and np.array_equal(a, b), f"{what}: {name}"
+    assert got.stats["hm_buckets"] == single.stats["hm_buckets"], what
+
+
+@pytest.mark.parametrize("how", ["shard2", "shard8", "multi4"])
+@pytest.mark.parametrize("name", sorted(CASES))
+def test_sharded_exports_of_golden_cases(built, name, how):
+    """Every golden case through the distributed finish with k-mers and hash-map layout exported: the graph
+    equals the compiled reference's (frequency saturation at 32765 included), the exports the one-device build's."""
+    case = CASES[name]
+    L, k, mf, mq = case["L"], case["k"], case["mf"], case["mq"]
+    gold = dict(np.load(os.path.join(GOLDEN_DIR, name + ".npz")))
+    gold["n_nodes"] = len(gold["first_pos"])
+    primary, secondary = make_inputs(case)
+    kw = dict(export_keys=True, hashmap_layout=True)
+    with GraphBuilder(L, k, mf, mq, **kw) as gb:
+        single = gb.build(primary, secondary)
+    assert_graph_equal(single, gold, f"{name} one device")
+    if how == "multi4":
+        with MultiBuilder(L, k, mf, mq, devices=[0] * 4, **kw) as mb:
+            got = mb.build(primary, secondary)
+    else:
+        got, _ = _sharded(primary, secondary, L, k, mf, mq, int(how[5:]), **kw)
+    assert_graph_equal(got, gold, f"{name} {how}")
+    _exports_equal(got, single, f"{name} {how}")
+
+
+def _four_way_input(k):
+    """Reads f1 + p + C + s + f2 for a random core k-mer C, every pair of flanking bases p, s and three pairs of
+    far flanks: C (and its reverse complement) has four successors and four predecessors, each seen in
+    several distinct reads."""
+    rng = np.random.default_rng(11)
+
+    def rnd(n):
+        return "".join("ACGT"[i] for i in rng.integers(0, 4, n))
+
+    core = rnd(k)
+    flanks = [(rnd(8), rnd(8)) for _ in range(3)]
+    reads = [f1 + p + core + s + f2 for f1, f2 in flanks for p in "ACGT" for s in "ACGT"]
+    return synth.records_from_reads(reads), np.zeros(1, np.uint8)
+
+
+@pytest.mark.parametrize("G", [2, 8])
+def test_sharded_fourth_successor_and_predecessor(built, G):
+    """A node's fourth edge does not fit its 32-byte row in the distributed finish and goes through the
+    overflow list."""
+    L, k, mf, mq = 30, 12, 2, 40
+    primary, secondary = _four_way_input(k)
+    want = loader.build(primary, secondary, L, k, mf, mq, kind="port")
+    assert np.count_nonzero((want["out_deg"] == 4) & (want["in_deg"] == 4)) >= 2
+    kw = dict(export_keys=True, hashmap_layout=True)
+    got, stats = _sharded(primary, secondary, L, k, mf, mq, G, **kw)
+    assert_graph_equal(got, want, f"four-way G={G}")
+    assert sum(s["n_pre_total"] for s in stats) == want["n_pre_total"]
+    with GraphBuilder(L, k, mf, mq, **kw) as gb:
+        single = gb.build(primary, secondary)
+    assert_graph_equal(single, want, "four-way one device")
+    _exports_equal(got, single, f"four-way G={G}")
