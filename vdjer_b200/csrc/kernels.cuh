@@ -53,6 +53,8 @@ constexpr int FLB = 6;           /* window flag bits: has-next, next base (2), t
 constexpr u32 CNT2_MASK = 0x00FFFFFFu; /* Slot2::count: N-free occurrences; bits 24..27: in-mask (base c preceded the k-mer
                                           in some read): the export probes only the predecessors that can exist */
 constexpr int CNT2_IN = 24;
+constexpr u32 CNT2_DISP = 1u << 28;    /* Slot2::count bit 28: some k-mer whose home is this slot was inserted further on
+                                          (set by t2_insert).  Clear: a k-mer that is not here is not in the table */
 constexpr u64 LOG_A = 1ull << 62, LOG_B = 1ull << 63;   /* those two flags in a log entry, above the stamp */
 constexpr int QSUM_SAT = 214;    /* MAX_QUAL_SUM-41, :356 */
 constexpr int MAX_LOG_RANKS = 11;/* ceil(214/20) */
@@ -165,7 +167,7 @@ struct Reads {
 struct Counters {
     u64 n_gated;
     u64 n_distinct;
-    u64 n_surv;
+    u64 n_surv_hot, n_surv_cold; /* survivors k_prune listed at the front / back of the survivor list */
     u64 n_hits;
     u64 n_nodes;
     u64 n_slow1, n_slow2; /* windows that took the slow path of pass 1 / pass 2 */
@@ -1424,6 +1426,31 @@ k_pass1(Pass1Args a, Geom g, Part pt) {
     if (lane == 0 && n_slow) atomicAdd(&a.ctr->n_slow1, (u64)n_slow);
 }
 
+/* Position of this thread's element in a global append-only array: warps sum their counts in
+ * shared memory and ONE global atomic per block reserves the block's range (a per-warp atomic on
+ * the single counter serialises: 400 k same-address atomics cost more than the scan itself).
+ * Must be called by all threads of the block; `take` = this thread appends one element to the array
+ * of `counter`, `take_b` (exclusive with take) one to the array of `counter_b`: two arrays cost one
+ * round of barriers, and their two atomics are in flight together. */
+__device__ __forceinline__ u64 block_append(bool take, u64 *counter, bool take_b = false, u64 *counter_b = nullptr) {
+    __shared__ u32 s_cnt[2];
+    __shared__ u64 s_base[2];
+    const u32 lane = threadIdx.x & 31, lt = (1u << lane) - 1;
+    if (threadIdx.x < 2) s_cnt[threadIdx.x] = 0;
+    __syncthreads();
+    const u32 ballot = __ballot_sync(0xFFFFFFFFu, take), ballot_b = __ballot_sync(0xFFFFFFFFu, take_b);
+    u32 wbase = 0, wbase_b = 0;
+    if (lane == 0 && ballot) wbase = atomicAdd(&s_cnt[0], (u32)__popc(ballot));
+    if (lane == 0 && ballot_b) wbase_b = atomicAdd(&s_cnt[1], (u32)__popc(ballot_b));
+    wbase = __shfl_sync(0xFFFFFFFFu, wbase, 0);
+    wbase_b = __shfl_sync(0xFFFFFFFFu, wbase_b, 0);
+    __syncthreads();
+    if (threadIdx.x == 0) s_base[0] = s_cnt[0] ? atomicAdd(counter, (u64)s_cnt[0]) : 0ull;
+    if (threadIdx.x == 32) s_base[1] = s_cnt[1] ? atomicAdd(counter_b, (u64)s_cnt[1]) : 0ull;
+    __syncthreads();
+    return take_b ? s_base[1] + wbase_b + __popc(ballot_b & lt) : s_base[0] + wbase + __popc(ballot & lt);
+}
+
 /* ------------------------------------------------------------------------------------------ */
 /* K3 k_prune = prune_pre_graph (:467-484) + is_base_quality_good (:454-465).                   */
 /* keep K iff frequency >= mf && hasMultipleUniqueReads && for all j qual_sums[j] >= mq.        */
@@ -1433,6 +1460,8 @@ k_pass1(Pass1Args a, Geom g, Part pt) {
 /* S_j >= T, T = min(mq, 214).  Every gated quality is >= 20, so S_j >= 20*(count-1): k-mers    */
 /* with 20*(count-1) >= T pass without looking at qualities; the others have count <= NB and    */
 /* their complete occurrence list is in the log.                                                */
+/* The survivors' slots go to a list that table 2 is built from: k-mers with a gated count >= hot */
+/* from the front, the others from the back, so that the hot ones can be inserted first.          */
 /* ------------------------------------------------------------------------------------------ */
 struct PruneArgs {
     Slot1 *table;
@@ -1441,10 +1470,15 @@ struct PruneArgs {
     u32 nb_ranks;
     Reads rd;
     int mf, T;
+    u32 hot;
+    u32 *surv;         /* [cap]: hot survivors' slots at [0, n_surv_hot), the others at [cap - n_surv_cold, cap) */
     Counters *ctr;
 };
 
-__global__ void __launch_bounds__(THREADS)
+/* 8 blocks per SM: the host's grid of 8 blocks per SM is resident at once.  Every iteration ends in a
+ * block-wide append; with fewer resident warps its barriers and atomic round trip are not hidden
+ * (configs[1] on a B200 at 1000 W: 0.83 ms at 6 blocks per SM and 40 registers, 0.52 ms at 8 and 32). */
+__global__ void __launch_bounds__(THREADS, 8)
 k_prune(PruneArgs a, Geom g) {
     /* lane = one slot; slots whose quality sums must be evaluated are then handled by the whole
      * warp: lane j owns k-mer positions j and j+32, so each occurrence's k quality bytes are one
@@ -1453,7 +1487,7 @@ k_prune(PruneArgs a, Geom g) {
     const u64 stride = (u64)gridDim.x * blockDim.x;
     const u64 n_iter = (a.cap + stride - 1) / stride;
     u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x;
-    u32 n_distinct = 0, n_surv = 0;
+    u32 n_distinct = 0;
     for (u64 itn = 0; itn < n_iter; itn++, i += stride) {
         u32 cnt = 0, cw = 0, head = NIL32;
         int lb_first = 0;
@@ -1517,40 +1551,40 @@ k_prune(PruneArgs a, Geom g) {
             const u32 any_bad = __ballot_sync(0xFFFFFFFFu, bad);
             if ((int)lane == b && any_bad) pass = false;
         }
-        if (pass) {
-            a.table[i].count = cw | CNT_SURV;
-            n_surv++;
-        }
+        if (pass) a.table[i].count = cw | CNT_SURV;
+        const bool hot = cnt >= a.hot;
+        const u64 at = block_append(pass && hot, &a.ctr->n_surv_hot, pass && !hot, &a.ctr->n_surv_cold);
+        if (pass) a.surv[hot ? at : a.cap - 1 - at] = (u32)i;
     }
-    for (int o = 16; o; o >>= 1) {
-        n_distinct += __shfl_xor_sync(0xFFFFFFFFu, n_distinct, o);
-        n_surv += __shfl_xor_sync(0xFFFFFFFFu, n_surv, o);
-    }
-    if (lane == 0) {
-        if (n_distinct) atomicAdd(&a.ctr->n_distinct, (u64)n_distinct);
-        if (n_surv) atomicAdd(&a.ctr->n_surv, (u64)n_surv);
-    }
+    for (int o = 16; o; o >>= 1) n_distinct += __shfl_xor_sync(0xFFFFFFFFu, n_distinct, o);
+    if (lane == 0 && n_distinct) atomicAdd(&a.ctr->n_distinct, (u64)n_distinct);
 }
 
 /* ------------------------------------------------------------------------------------------ */
 /* survivor table (pass-2 membership + per-node reductions), partitioned like table 1           */
 /* ------------------------------------------------------------------------------------------ */
+/* inserts from the home slot idx and marks the home CNT2_DISP when another k-mer holds it.  The count
+ * word of a slot is only ever OR-ed or added to (k_init_table2 zeroes it), so the mark survives the
+ * seeding of the k-mer that holds the home. */
 __device__ __forceinline__ u64 t2_insert(Slot2 *t, u64 cap, u64 idx, u64 lo, u64 hi) {
     for (u32 probe = 0; probe < MAX_PROBE; probe++) {
         u64 o0, o1;
         cas128(&t[idx], EMPTY64, EMPTY64, lo, hi, o0, o1);
         if ((o0 == EMPTY64 && o1 == EMPTY64) || (o0 == lo && o1 == hi)) return idx;
+        if (probe == 0) atomicOr(&t[idx].count, CNT2_DISP);
         if (++idx == cap) idx = 0;
     }
     return INF64;
 }
-/* linear probe from idx; returns slot index or INF64; fills words 2,3 of the hot sector */
-__device__ __forceinline__ u64 t2_probe_from(const Slot2 *t, u64 cap, u64 idx, u64 lo, u64 hi, u64 &q2, u64 &q3) {
+/* linear probe from idx; returns slot index or INF64; fills words 2,3 of the hot sector.  home: idx is
+ * the k-mer's home slot, so another k-mer there without CNT2_DISP ends the search */
+__device__ __forceinline__ u64 t2_probe_from(const Slot2 *t, u64 cap, u64 idx, u64 lo, u64 hi, u64 &q2, u64 &q3, bool home) {
     for (u32 probe = 0; probe < MAX_PROBE; probe++) {
         u64 q0, q1;
         ld_sector(&t[idx], q0, q1, q2, q3);
         if (q0 == lo && q1 == hi) return idx;
         if (q0 == EMPTY64 && q1 == EMPTY64) return INF64;
+        if (home && probe == 0 && !((u32)q2 & CNT2_DISP)) return INF64;
         if (++idx == cap) idx = 0;
     }
     return INF64;
@@ -1563,44 +1597,25 @@ __device__ __forceinline__ u32 t2_home(const Part &pt, const Geom &g, u64 lo, u6
     return slot_in(h, ut.z, ut.w);
 }
 __device__ __forceinline__ u64 t2_find(const Slot2 *t, u64 cap, const Part &pt, const Geom &g, u64 lo, u64 hi, u64 &q2, u64 &q3) {
-    return t2_probe_from(t, cap, t2_home(pt, g, lo, hi), lo, hi, q2, q3);
+    return t2_probe_from(t, cap, t2_home(pt, g, lo, hi), lo, hi, q2, q3, true);
 }
 
+/* inserts the survivors whose table-1 slots are surv[0, n).  The host launches it on the hot part of
+ * k_prune's list first: a k-mer inserted early is more likely to sit at its home slot, where pass 2
+ * finds it with one probe, and most windows are windows of hot k-mers. */
 __global__ void __launch_bounds__(THREADS)
-k_build_table2(const Slot1 *t1, u64 cap1, Slot2 *t2, u64 cap2, Geom g, Part pt, Counters *ctr) {
+k_build_table2(const Slot1 *t1, const u32 *surv, u64 n, Slot2 *t2, u64 cap2, Geom g, Part pt, Counters *ctr) {
     u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x, stride = (u64)gridDim.x * blockDim.x;
-    for (; i < cap1; i += stride) {
+    for (; i < n; i += stride) {
         u64 q0, q1, q2, q3;
-        ld_sector(&t1[i], q0, q1, q2, q3);
-        if (q0 == EMPTY64 && q1 == EMPTY64) continue;
-        if (!((u32)q2 & CNT_SURV)) continue;
+        ld_sector(&t1[surv[i]], q0, q1, q2, q3);
         /* (the slice a table-1 slot lies in says nothing: probing runs past slice ends) */
         const u64 at = t2_insert(t2, cap2, t2_home(pt, g, q0, q1), q0, q1);
         if (at == INF64) { atomicExch(&ctr->overflow, 3u); continue; }
         /* the gated occurrences are N-free occurrences: seed node->frequency with them */
         const u32 cnt = ((u32)q2 & CNT_MASK) + 1;
-        t2[at].count = cnt > CNT_CAP ? CNT_CAP : cnt;
+        atomicOr(&t2[at].count, cnt > CNT_CAP ? CNT_CAP : cnt);
     }
-}
-
-/* Position of this thread's element in a global append-only array: warps sum their counts in
- * shared memory and ONE global atomic per block reserves the block's range (a per-warp atomic on
- * the single counter serialises: 400 k same-address atomics cost more than the scan itself).
- * Must be called by all threads of the block; `take` = this thread appends one element. */
-__device__ __forceinline__ u64 block_append(bool take, u64 *counter) {
-    __shared__ u32 s_cnt;
-    __shared__ u64 s_base;
-    const u32 lane = threadIdx.x & 31;
-    if (threadIdx.x == 0) s_cnt = 0;
-    __syncthreads();
-    const u32 ballot = __ballot_sync(0xFFFFFFFFu, take);
-    u32 wbase = 0;
-    if (lane == 0 && ballot) wbase = atomicAdd(&s_cnt, (u32)__popc(ballot));
-    wbase = __shfl_sync(0xFFFFFFFFu, wbase, 0);
-    __syncthreads();
-    if (threadIdx.x == 0) s_base = s_cnt ? atomicAdd(counter, (u64)s_cnt) : 0ull;
-    __syncthreads();
-    return s_base + wbase + __popc(ballot & ((1u << lane) - 1));
 }
 
 /* Sharded build: a device's survivors as dense Slot2 records (sent to the finishing device), and
@@ -1633,7 +1648,8 @@ k_table2_from_records(const Slot2 *rec, u64 n, Slot2 *t2, u64 cap2, Geom g, Part
         const u64 at = t2_insert(t2, cap2, t2_home(pt, g, q0, q1), q0, q1);
         if (at == INF64) { atomicExch(&ctr->overflow, 3u); continue; }
         Slot2 *o = t2 + at;
-        o->count = (u32)q2; o->rank = 0; o->first_any = q3;
+        atomicOr(&o->count, (u32)q2 & ~CNT2_DISP);   /* the record's mark is about the table it was compacted from */
+        o->rank = 0; o->first_any = q3;
         st_sector(reinterpret_cast<char *>(o) + 32, r0, r1, r2, r3);
     }
 }
@@ -1787,7 +1803,8 @@ k_pass2(Pass2Args a, Geom g, Part pt) {
                     of[u] = ld_ca_u64(&a.table[idx[u]].out_first[(fl[u] >> 1) & 3u]);
                 }
             }
-            /* B: hit at home -> reductions; empty home -> the k-mer did not survive; otherwise queue.
+            /* B: hit at home -> reductions; home without CNT2_DISP (empty, or nothing was displaced from it;
+             * q2 is zero for a window with an N) -> the k-mer did not survive; otherwise queue.
              * node->frequency counts every N-free occurrence; the gated ones were already counted by
              * pass 1 (k_build_table2 seeds count with them), so only ungated windows add to it. */
 #pragma unroll
@@ -1795,14 +1812,13 @@ k_pass2(Pass2Args a, Geom g, Part pt) {
                 const bool valid = idx[u] != NIL32;
                 const bool ungated = !((fl[u] >> FLB) & 1u);
                 const bool hit = valid && q0[u] == lo[u] && q1[u] == hi[u];
-                const bool empty = q0[u] == EMPTY64 && q1[u] == EMPTY64;
                 if (hit) {
                     pass2_update(a.table + idx[u], ungated, q2[u], q3[u], of[u], (edges >> u) & 1u, (fl[u] >> 1) & 3u, stamp[u],
                                  (fl[u] >> 8) & 0xFFu, fl[u]);
                     n_hits++;
                     n_hits_u += ungated;
                 }
-                qn = q.push_lazy(qn, valid && !hit && !empty, lo[u], idx[u] | (ungated ? 0x80000000u : 0u), [&](u64 &t1, u64 &t2) {
+                qn = q.push_lazy(qn, !hit && (q2[u] & CNT2_DISP), lo[u], idx[u] | (ungated ? 0x80000000u : 0u), [&](u64 &t1, u64 &t2) {
                     pack_tuple<WIDE>(pt, hi[u], fl[u] & ((1u << FLB) - 1), 0u, stamp[u], t1, t2);
                 });
             }
@@ -1927,7 +1943,7 @@ k_export(ExportArgs a, Geom g, Part pt) {
         if (tf == INF64) continue;
         u64 slo, shi, q2, q3;
         kmer_succ(lo, hi, c, g.k, slo, shi);
-        u64 idx = t2_probe_from(a.table, a.cap, t2_home_in(pt, pt.flat ? 0u : nm.succ_bucket(c, g), slo, shi), slo, shi, q2, q3);
+        u64 idx = t2_probe_from(a.table, a.cap, t2_home_in(pt, pt.flat ? 0u : nm.succ_bucket(c, g), slo, shi), slo, shi, q2, q3, true);
         if (idx == INF64) continue;
         tt[n] = tf; vv[n] = (u32)(q2 >> 32); n++;
     }
@@ -1942,7 +1958,7 @@ k_export(ExportArgs a, Geom g, Part pt) {
         if (!((in_mask >> c) & 1u)) continue;   /* never seen after base c: c+K[:-1] -> K was never linked */
         u64 plo, phi, q2, q3;
         kmer_pred(lo, hi, c, g.kmask_lo, g.kmask_hi, plo, phi);
-        u64 idx = t2_probe_from(a.table, a.cap, t2_home_in(pt, pt.flat ? 0u : nm.pred_bucket(c, g), plo, phi), plo, phi, q2, q3);
+        u64 idx = t2_probe_from(a.table, a.cap, t2_home_in(pt, pt.flat ? 0u : nm.pred_bucket(c, g), plo, phi), plo, phi, q2, q3, true);
         if (idx == INF64) continue;
         u64 tf = a.table[idx].out_first[last];
         if (tf == INF64) continue;
@@ -2056,7 +2072,7 @@ k_export_dist(ExportDistArgs a, const __grid_constant__ PeerTables pt, Geom g, c
         u64 slo, shi, q2, q3;
         kmer_succ(lo, hi, c, g.k, slo, shi);
         const u32 d = __ldg(pt.owner + (nm.succ_bucket(c, g) >> pt.ushift));
-        const u64 idx = t2_probe_from(pt.table[d], pt.len[d], slot_in(hash_slot(slo, shi), 0u, pt.len[d]), slo, shi, q2, q3);
+        const u64 idx = t2_probe_from(pt.table[d], pt.len[d], slot_in(hash_slot(slo, shi), 0u, pt.len[d]), slo, shi, q2, q3, true);
         if (idx == INF64) continue;
         tt[n] = tf; vv[n] = (u32)(q2 >> 32); n++;
     }
@@ -2070,7 +2086,7 @@ k_export_dist(ExportDistArgs a, const __grid_constant__ PeerTables pt, Geom g, c
         u64 plo, phi, q2, q3;
         kmer_pred(lo, hi, c, g.kmask_lo, g.kmask_hi, plo, phi);
         const u32 d = __ldg(pt.owner + (nm.pred_bucket(c, g) >> pt.ushift));
-        const u64 idx = t2_probe_from(pt.table[d], pt.len[d], slot_in(hash_slot(plo, phi), 0u, pt.len[d]), plo, phi, q2, q3);
+        const u64 idx = t2_probe_from(pt.table[d], pt.len[d], slot_in(hash_slot(plo, phi), 0u, pt.len[d]), plo, phi, q2, q3, true);
         if (idx == INF64) continue;
         const u64 tf = ld_cg_u64(&pt.table[d][idx].out_first[last]);
         if (tf == INF64) continue;
@@ -2341,9 +2357,9 @@ k_query(QueryArgs a, Geom g, Part pt) {
         for (int b = 0; b < BATCH; b++) {
             if (!live[b]) continue;
             bool hit = k0[b] == lo[b] && k1[b] == hi[b];
-            if (!hit && !(k0[b] == EMPTY64 && k1[b] == EMPTY64)) {
+            if (!hit && ((u32)q2[b] & CNT2_DISP)) {   /* (an empty home has no mark) */
                 const u64 from = idx[b] + 1 == a.cap ? 0 : idx[b] + 1;
-                hit = t2_probe_from(a.table, a.cap, from, lo[b], hi[b], q2[b], q3[b]) != INF64;
+                hit = t2_probe_from(a.table, a.cap, from, lo[b], hi[b], q2[b], q3[b], false) != INF64;
             }
             if (hit) { rank[b] = (u32)(q2[b] >> 32); n_found++; }
         }

@@ -301,7 +301,7 @@ struct vdjgraph_ctx {
 
     DevBuf d_bad, d_bases, d_good, d_valid, d_hiq, d_qual, d_strand;
     PinBuf h_bad;
-    DevBuf d_t1, d_log, d_t2, d_hll, d_ctr, d_hist, d_cursor, d_tuples, d_utab;
+    DevBuf d_t1, d_surv, d_log, d_t2, d_hll, d_ctr, d_hist, d_cursor, d_tuples, d_utab;
     DevBuf d_keys[2], d_vals[2], d_cub;
     NodeArrays nodes;
     DevBuf d_pre_klo, d_pre_khi, d_pre_freq, d_pre_n;
@@ -964,7 +964,7 @@ int run_plan(vdjgraph_ctx *c, const uint64_t *hist_all, const uint8_t *hll) {
         const bool merged = G * sh.S > 1;
         for (size_t i = 0; i < load_rnd.size(); i++) {
             const double cap1_dev = est_rnd[i];
-            const double tables = cap1_dev * sizeof(Slot1)
+            const double tables = cap1_dev * (sizeof(Slot1) + sizeof(u32))   /* table 1 and k_prune's survivor list */
                                 + std::min((double)gated_rnd[i], cap1_dev * load1 / 1.15 * 1.3) * NBq * 8.0
                                 + nodes / ((double)G * sh.S) * 4.0 * sizeof(Slot2);
             /* the finish.  One device, several rounds: merged table over all survivor records, sort buffers,
@@ -1159,6 +1159,7 @@ int run_passes(vdjgraph_ctx *c) {
         if (NB == 0) log_cap = 1;
         if (log_cap > 0xFFFFFFF0ull) return fail(VDJGRAPH_ERR_TOO_MANY_NODES, "occurrence log would need %llu blocks", (unsigned long long)log_cap);
         if ((rc = c->d_t1.ensure(cap1 * sizeof(Slot1)))) return rc;
+        if ((rc = c->d_surv.ensure(cap1 * sizeof(u32)))) return rc;
         if ((rc = c->d_log.ensure(log_cap * (uint64_t)std::max(NB, 1) * sizeof(uint64_t)))) return rc;
         c->cap1 = cap1; c->log_cap = (uint32_t)log_cap;
         memcpy(ut, sh.utab.data(), sh.NU * sizeof(UnitTab));
@@ -1180,6 +1181,7 @@ int run_passes(vdjgraph_ctx *c) {
         PruneArgs ap;
         ap.table = c->d_t1.as<Slot1>(); ap.cap = cap1; ap.log = c->d_log.as<u64>(); ap.nb_ranks = (uint32_t)NB;
         ap.rd = rd; ap.mf = c->prm.min_node_freq; ap.T = T; ap.ctr = d_ctr;
+        ap.hot = (u32)std::min<double>(CNT_CAP + 1, std::max(1.0, env_double("VDJGRAPH_HOT2", 32))); ap.surv = c->d_surv.as<u32>();
         k_prune<<<grid_flat, THREADS, 0, s>>>(ap, g);
         CK(cudaEventRecord(c->ev[EV_PRUNE_END], s));
         res.kernel_launches += 3;
@@ -1195,7 +1197,7 @@ int run_passes(vdjgraph_ctx *c) {
         if (h_ctr->internal) return fail(VDJGRAPH_ERR_INTERNAL, "occurrence log inconsistent (code %u)", h_ctr->internal);
         break;
     }
-    const uint64_t n_surv = h_ctr->n_surv;
+    const uint64_t n_hot = h_ctr->n_surv_hot, n_surv = n_hot + h_ctr->n_surv_cold;
     res.n_slow1 += h_ctr->n_slow1;          /* sums over the rounds (zeroed by run_plan) */
     res.n_pre_total += h_ctr->n_distinct;
     res.n_pre += n_surv;
@@ -1226,7 +1228,10 @@ int run_passes(vdjgraph_ctx *c) {
     CK(cudaMemcpyAsync(c->d_utab.p, ut, sh.NU * sizeof(UnitTab), cudaMemcpyHostToDevice, s));
     CK(cudaEventRecord(c->ev[EV_TABLE2], s));
     k_init_table2<<<grid_flat, THREADS, 0, s>>>(c->d_t2.as<Slot2>(), cap2);
-    k_build_table2<<<grid_flat, THREADS, 0, s>>>(c->d_t1.as<Slot1>(), cap1, c->d_t2.as<Slot2>(), cap2, g, pt, d_ctr);
+    /* the hot part of k_prune's survivor list, then the rest (see k_build_table2) */
+    k_build_table2<<<grid_flat, THREADS, 0, s>>>(c->d_t1.as<Slot1>(), c->d_surv.as<u32>(), n_hot, c->d_t2.as<Slot2>(), cap2, g, pt, d_ctr);
+    k_build_table2<<<grid_flat, THREADS, 0, s>>>(c->d_t1.as<Slot1>(), c->d_surv.as<u32>() + (cap1 - (n_surv - n_hot)), n_surv - n_hot,
+                                                 c->d_t2.as<Slot2>(), cap2, g, pt, d_ctr);
     CK(cudaEventRecord(c->ev[EV_PASS2], s));
     Pass2Args a2;
     a2.runs = c->d_tuples.as<u64>();
@@ -1234,7 +1239,7 @@ int run_passes(vdjgraph_ctx *c) {
     if (pt.wide) k_pass2<true><<<grid_p2, THREADS, smem_q, s>>>(a2, g, pt);
     else k_pass2<false><<<grid_p2, THREADS, smem_q, s>>>(a2, g, pt);
     CK(cudaEventRecord(c->ev[EV_PASS2_END], s));
-    res.kernel_launches += 3;
+    res.kernel_launches += 4;
     CK(cudaGetLastError());
     res.table1_slots = cap1; res.table2_slots = cap2;
     if (sh.merged()) {
@@ -1344,7 +1349,7 @@ int run_finish(vdjgraph_ctx *c) {
         const double free_mb = env_double("VDJGRAPH_FREE_TABLES_MB", -1.0);
         if (free_mb >= 0 && (double)(cap2 * sizeof(Slot2)) > free_mb * 1048576.0) {
             CK(cudaStreamSynchronize(s));
-            c->d_t1.release(); c->d_log.release(); c->d_t2.release();
+            c->d_t1.release(); c->d_surv.release(); c->d_log.release(); c->d_t2.release();
         }
         pt.flat = 1; pt.flat_len = (u32)cap2;
         if ((rc = c->d_t2m.ensure(cap2 * sizeof(Slot2)))) return rc;
