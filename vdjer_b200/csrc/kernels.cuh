@@ -1576,28 +1576,32 @@ __device__ __forceinline__ u64 t2_insert(Slot2 *t, u64 cap, u64 idx, u64 lo, u64
     }
     return INF64;
 }
-/* linear probe from idx; returns slot index or INF64; fills words 2,3 of the hot sector.  home: idx is
- * the k-mer's home slot, so another k-mer there without CNT2_DISP ends the search */
-__device__ __forceinline__ u64 t2_probe_from(const Slot2 *t, u64 cap, u64 idx, u64 lo, u64 hi, u64 &q2, u64 &q3, bool home) {
+/* q2 = word 2 of a k-mer's home slot that holds another k-mer: can the k-mer be further on? */
+__device__ __forceinline__ bool home_displaced(u64 q2) { return (u32)q2 & CNT2_DISP; }
+/* linear probe from idx; returns slot index or INF64; fills word 2 of the hot sector.  home: idx is
+ * the k-mer's home slot, so another k-mer there ends the search unless home_displaced */
+__device__ __forceinline__ u64 t2_probe_from(const Slot2 *t, u64 cap, u64 idx, u64 lo, u64 hi, u64 &q2, bool home) {
     for (u32 probe = 0; probe < MAX_PROBE; probe++) {
-        u64 q0, q1;
+        u64 q0, q1, q3;
         ld_sector(&t[idx], q0, q1, q2, q3);
         if (q0 == lo && q1 == hi) return idx;
         if (q0 == EMPTY64 && q1 == EMPTY64) return INF64;
-        if (home && probe == 0 && !((u32)q2 & CNT2_DISP)) return INF64;
+        if (home && probe == 0 && !home_displaced(q2)) return INF64;
         if (++idx == cap) idx = 0;
     }
     return INF64;
 }
-/* home slot of an arbitrary k-mer in table 2: in the slice of its hash unit, or anywhere in a flat (merged) table */
-__device__ __forceinline__ u32 t2_home(const Part &pt, const Geom &g, u64 lo, u64 hi) {
+/* home slot in table 2 of a k-mer: in the slice of its hash unit (bucket() = its minimizer bucket), or anywhere in a
+ * flat (merged) table, where bucket() is not called */
+template <class Bucket>
+__device__ __forceinline__ u32 t2_home_in(const Part &pt, Bucket bucket, u64 lo, u64 hi) {
     const u32 h = hash_slot(lo, hi);
     if (pt.flat) return slot_in(h, 0u, pt.flat_len);
-    const uint4 ut = __ldg(reinterpret_cast<const uint4 *>(pt.ut + (kmer_bucket_of(lo, hi, g.span, g.mmask) >> pt.ushift)));
+    const uint4 ut = __ldg(reinterpret_cast<const uint4 *>(pt.ut + (bucket() >> pt.ushift)));
     return slot_in(h, ut.z, ut.w);
 }
-__device__ __forceinline__ u64 t2_find(const Slot2 *t, u64 cap, const Part &pt, const Geom &g, u64 lo, u64 hi, u64 &q2, u64 &q3) {
-    return t2_probe_from(t, cap, t2_home(pt, g, lo, hi), lo, hi, q2, q3, true);
+__device__ __forceinline__ u32 t2_home(const Part &pt, const Geom &g, u64 lo, u64 hi) {
+    return t2_home_in(pt, [&] { return kmer_bucket_of(lo, hi, g.span, g.mmask); }, lo, hi);
 }
 
 /* inserts the survivors whose table-1 slots are surv[0, n).  The host launches it on the hot part of
@@ -1618,8 +1622,8 @@ k_build_table2(const Slot1 *t1, const u32 *surv, u64 n, Slot2 *t2, u64 cap2, Geo
     }
 }
 
-/* Sharded build: a device's survivors as dense Slot2 records (sent to the finishing device), and
- * the finishing device's table over the records of all devices. */
+/* Sharded or multi-round build: a device's survivors as dense Slot2 records, appended round after round,
+ * and the finish's flat table over the records of all rounds of this device. */
 __global__ void __launch_bounds__(THREADS)
 k_compact_table2(const Slot2 *t, u64 cap, Slot2 *out, u64 *n_out) {
     u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x, stride = (u64)gridDim.x * blockDim.x;
@@ -1818,7 +1822,7 @@ k_pass2(Pass2Args a, Geom g, Part pt) {
                     n_hits++;
                     n_hits_u += ungated;
                 }
-                qn = q.push_lazy(qn, !hit && (q2[u] & CNT2_DISP), lo[u], idx[u] | (ungated ? 0x80000000u : 0u), [&](u64 &t1, u64 &t2) {
+                qn = q.push_lazy(qn, !hit && home_displaced(q2[u]), lo[u], idx[u] | (ungated ? 0x80000000u : 0u), [&](u64 &t1, u64 &t2) {
                     pack_tuple<WIDE>(pt, hi[u], fl[u] & ((1u << FLB) - 1), 0u, stamp[u], t1, t2);
                 });
             }
@@ -1889,13 +1893,67 @@ struct NeighbourMini {
         return mini_bucket(min(head, mini_hash(((x_first << 2) | c) & g.mmask)));
     }
 };
-/* home slot in table 2 of a k-mer whose bucket is known */
-__device__ __forceinline__ u32 t2_home_in(const Part &pt, u32 bucket, u64 lo, u64 hi) {
-    const u32 h = hash_slot(lo, hi);
-    if (pt.flat) return slot_in(h, 0u, pt.flat_len);
-    const uint4 ut = __ldg(reinterpret_cast<const uint4 *>(pt.ut + (bucket >> pt.ushift)));
-    return slot_in(h, ut.z, ut.w);
+
+/* out = v[0, n) in descending order of t, NIL32 beyond n */
+__device__ __forceinline__ void sort_desc4(u64 (&t)[4], u32 (&v)[4], int n, u32 (&out)[4]) {
+    for (int a = 1; a < n; a++)
+        for (int b = a; b > 0 && t[b] > t[b - 1]; b--) {
+            u64 x = t[b]; t[b] = t[b - 1]; t[b - 1] = x;
+            u32 y = v[b]; v[b] = v[b - 1]; v[b - 1] = y;
+        }
+    for (int e = 0; e < 4; e++) out[e] = e < n ? v[e] : NIL32;
 }
+struct Edges { int n_out, n_in; u32 succ[4], pred[4]; };   /* NIL32 beyond the degrees */
+
+/* The edge lists of the node with key (lo, hi), count word cw and out_first words of[4], in the reference's order.
+ * Lookup: buckets() (may find ask for a bucket?), find(bucket, lo, hi, q2) = a neighbour's slot or null (bucket() =
+ * its minimizer bucket, q2 = word 2: its rank above bit 32), out_first(slot, c). */
+template <class Lookup>
+__device__ __forceinline__ Edges node_edges(const Lookup &lk, const Geom &g, u64 lo, u64 hi, u32 cw, const u64 *of) {
+    Edges e;
+    u64 tt[4]; u32 vv[4];
+    NeighbourMini nm;
+    if (lk.buckets()) nm.scan(lo, hi, g);     /* the buckets of all eight neighbours from one scan of the k-mer */
+    /* toNodes: successors K[1:]+c that survived, newest first-seen at the head (:223-229) */
+    int n = 0;
+#pragma unroll 1   /* the probes are serial anyway (ld_sector is volatile); unrolled, k_export spills */
+    for (u32 c = 0; c < 4; c++) {
+        const u64 tf = of[c];
+        if (tf == INF64) continue;
+        u64 slo, shi, q2;
+        kmer_succ(lo, hi, c, g.k, slo, shi);
+        if (!lk.find([&] { return nm.succ_bucket(c, g); }, slo, shi, q2)) continue;
+        tt[n] = tf; vv[n] = (u32)(q2 >> 32); n++;
+    }
+    sort_desc4(tt, vv, n, e.succ); e.n_out = n;
+    /* fromNodes: predecessors c+K[:-1] that survived and were seen followed by K's last base;
+     * the edge P->K was first linked at P.out_first[last(K)] + 1 (:231-236) */
+    n = 0;
+    const u32 last = kmer_last(lo, hi, g.k), in_mask = (cw >> CNT2_IN) & 15u;
+    for (u32 c = 0; c < 4; c++) {
+        if (!((in_mask >> c) & 1u)) continue;   /* never seen after base c: c+K[:-1] -> K was never linked */
+        u64 plo, phi, q2;
+        kmer_pred(lo, hi, c, g.kmask_lo, g.kmask_hi, plo, phi);
+        const Slot2 *p = lk.find([&] { return nm.pred_bucket(c, g); }, plo, phi, q2);
+        if (!p) continue;
+        const u64 tf = lk.out_first(p, last);
+        if (tf == INF64) continue;
+        tt[n] = tf; vv[n] = (u32)(q2 >> 32); n++;
+    }
+    sort_desc4(tt, vv, n, e.pred); e.n_in = n;
+    return e;
+}
+
+/* neighbours in this device's table: sliced by hash unit, or flat (merged), where no bucket is needed */
+struct LocalTable {
+    const Slot2 *table; u64 cap; Part pt;
+    __device__ __forceinline__ bool buckets() const { return !pt.flat; }
+    template <class Bucket> __device__ __forceinline__ const Slot2 *find(Bucket bucket, u64 lo, u64 hi, u64 &q2) const {
+        const u64 idx = t2_probe_from(table, cap, t2_home_in(pt, bucket, lo, hi), lo, hi, q2, true);
+        return idx == INF64 ? nullptr : table + idx;
+    }
+    __device__ __forceinline__ u64 out_first(const Slot2 *s, u32 c) const { return s->out_first[c]; }
+};
 
 struct ExportArgs {
     const Slot2 *table;
@@ -1910,14 +1968,6 @@ struct ExportArgs {
     u64 *kmer_lo, *kmer_hi; /* may be null */
 };
 
-__device__ __forceinline__ void sort_desc4(u64 (&t)[4], u32 (&v)[4], int n) {
-    for (int a = 1; a < n; a++)
-        for (int b = a; b > 0 && t[b] > t[b - 1]; b--) {
-            u64 x = t[b]; t[b] = t[b - 1]; t[b - 1] = x;
-            u32 y = v[b]; v[b] = v[b - 1]; v[b - 1] = y;
-        }
-}
-
 /* one thread per node, in creation order (coalesced result rows).  Measured and rejected: walking
  * the table in slot order with a bucket-sliced merged table, to keep the <= 8 neighbour lookups of
  * a node inside one L2-resident slice (its neighbours mostly share its minimizer): the scattered
@@ -1929,44 +1979,14 @@ k_export(ExportArgs a, Geom g, Part pt) {
     if (i >= a.n) return;
     const Slot2 *s = a.table + a.vals[i];
     const u64 lo = s->klo, hi = s->khi;
-    const u32 cw = s->count, cnt = cw & CNT2_MASK, in_mask = (cw >> CNT2_IN) & 15u;
+    const u32 cw = s->count, cnt = cw & CNT2_MASK;
     a.first_pos[i] = a.keys[i];
     a.frequency[i] = (u16)(cnt > CNT_CAP ? CNT_CAP : cnt);
     if (a.kmer_lo) { a.kmer_lo[i] = lo; a.kmer_hi[i] = hi; }
-    u64 tt[4]; u32 vv[4];
-    NeighbourMini nm;
-    if (!pt.flat) nm.scan(lo, hi, g);     /* the buckets of all eight neighbours from one scan of the k-mer */
-    /* toNodes: successors K[1:]+c that survived, newest first-seen at the head (:223-229) */
-    int n = 0;
-    for (u32 c = 0; c < 4; c++) {
-        u64 tf = s->out_first[c];
-        if (tf == INF64) continue;
-        u64 slo, shi, q2, q3;
-        kmer_succ(lo, hi, c, g.k, slo, shi);
-        u64 idx = t2_probe_from(a.table, a.cap, t2_home_in(pt, pt.flat ? 0u : nm.succ_bucket(c, g), slo, shi), slo, shi, q2, q3, true);
-        if (idx == INF64) continue;
-        tt[n] = tf; vv[n] = (u32)(q2 >> 32); n++;
-    }
-    sort_desc4(tt, vv, n);
-    a.out_deg[i] = (u8)n;
-    for (int e = 0; e < 4; e++) a.out_succ[i * 4 + e] = e < n ? vv[e] : NIL32;
-    /* fromNodes: predecessors c+K[:-1] that survived and were seen followed by K's last base;
-     * the edge P->K was first linked at P.out_first[last(K)] + 1 (:231-236) */
-    n = 0;
-    const u32 last = kmer_last(lo, hi, g.k);
-    for (u32 c = 0; c < 4; c++) {
-        if (!((in_mask >> c) & 1u)) continue;   /* never seen after base c: c+K[:-1] -> K was never linked */
-        u64 plo, phi, q2, q3;
-        kmer_pred(lo, hi, c, g.kmask_lo, g.kmask_hi, plo, phi);
-        u64 idx = t2_probe_from(a.table, a.cap, t2_home_in(pt, pt.flat ? 0u : nm.pred_bucket(c, g), plo, phi), plo, phi, q2, q3, true);
-        if (idx == INF64) continue;
-        u64 tf = a.table[idx].out_first[last];
-        if (tf == INF64) continue;
-        tt[n] = tf; vv[n] = (u32)(q2 >> 32); n++;
-    }
-    sort_desc4(tt, vv, n);
-    a.in_deg[i] = (u8)n;
-    for (int e = 0; e < 4; e++) a.in_pred[i * 4 + e] = e < n ? vv[e] : NIL32;
+    const Edges ed = node_edges(LocalTable{a.table, a.cap, pt}, g, lo, hi, cw, s->out_first);
+    a.out_deg[i] = (u8)ed.n_out;
+    a.in_deg[i] = (u8)ed.n_in;
+    for (int e = 0; e < 4; e++) { a.out_succ[i * 4 + e] = ed.succ[e]; a.in_pred[i * 4 + e] = ed.pred[e]; }
 }
 
 /* ------------------------------------------------------------------------------------------ */
@@ -1997,11 +2017,19 @@ struct RowSink {
     ulonglong2 *kmers; /* [n] or null */
 };
 
+/* neighbours in the flat table of the device that owns their bucket (node_edges' Lookup) */
 struct PeerTables {
     const Slot2 *table[MAX_DEV];   /* every device's flat survivor table (own: local pointer) */
     u32 len[MAX_DEV];
     const u8 *owner;               /* [hash units] owning device */
     u32 ushift;
+    __device__ __forceinline__ bool buckets() const { return true; }
+    template <class Bucket> __device__ __forceinline__ const Slot2 *find(Bucket bucket, u64 lo, u64 hi, u64 &q2) const {
+        const u32 d = __ldg(owner + (bucket() >> ushift));
+        const u64 idx = t2_probe_from(table[d], len[d], slot_in(hash_slot(lo, hi), 0u, len[d]), lo, hi, q2, true);
+        return idx == INF64 ? nullptr : table[d] + idx;
+    }
+    __device__ __forceinline__ u64 out_first(const Slot2 *s, u32 c) const { return ld_cg_u64(&s->out_first[c]); }
 };
 struct KeySegs {
     u64 off[MAX_DEV + 1];          /* device d's sorted stamps are all_keys[off[d] .. off[d+1]) */
@@ -2060,47 +2088,15 @@ k_export_dist(ExportDistArgs a, const __grid_constant__ PeerTables pt, Geom g, c
     if (i >= a.n) return;
     const Slot2 *s = pt.table[a.self] + a.vals[i];
     const u64 lo = s->klo, hi = s->khi;
-    const u32 cw = s->count, cnt = cw & CNT2_MASK, in_mask = (cw >> CNT2_IN) & 15u;
-    u64 tt[4]; u32 vv[4];
-    NeighbourMini nm;
-    nm.scan(lo, hi, g);
-    u32 succ[4], pred[4];
-    int n = 0;
-    for (u32 c = 0; c < 4; c++) {
-        const u64 tf = s->out_first[c];
-        if (tf == INF64) continue;
-        u64 slo, shi, q2, q3;
-        kmer_succ(lo, hi, c, g.k, slo, shi);
-        const u32 d = __ldg(pt.owner + (nm.succ_bucket(c, g) >> pt.ushift));
-        const u64 idx = t2_probe_from(pt.table[d], pt.len[d], slot_in(hash_slot(slo, shi), 0u, pt.len[d]), slo, shi, q2, q3, true);
-        if (idx == INF64) continue;
-        tt[n] = tf; vv[n] = (u32)(q2 >> 32); n++;
-    }
-    sort_desc4(tt, vv, n);
-    const int n_out = n;
-    for (int e = 0; e < 4; e++) succ[e] = e < n ? vv[e] : NIL32;
-    n = 0;
-    const u32 last = kmer_last(lo, hi, g.k);
-    for (u32 c = 0; c < 4; c++) {
-        if (!((in_mask >> c) & 1u)) continue;
-        u64 plo, phi, q2, q3;
-        kmer_pred(lo, hi, c, g.kmask_lo, g.kmask_hi, plo, phi);
-        const u32 d = __ldg(pt.owner + (nm.pred_bucket(c, g) >> pt.ushift));
-        const u64 idx = t2_probe_from(pt.table[d], pt.len[d], slot_in(hash_slot(plo, phi), 0u, pt.len[d]), plo, phi, q2, q3, true);
-        if (idx == INF64) continue;
-        const u64 tf = ld_cg_u64(&pt.table[d][idx].out_first[last]);
-        if (tf == INF64) continue;
-        tt[n] = tf; vv[n] = (u32)(q2 >> 32); n++;
-    }
-    sort_desc4(tt, vv, n);
-    for (int e = 0; e < 4; e++) pred[e] = e < n ? vv[e] : NIL32;
+    const u32 cw = s->count, cnt = cw & CNT2_MASK;
+    const Edges e = node_edges(pt, g, lo, hi, cw, s->out_first);
     const u32 id = a.gid[i];
-    const u64 w0 = a.keys[i] | ((u64)(cnt > CNT_CAP ? CNT_CAP : cnt) << 40) | ((u64)n_out << 56) | ((u64)n << 59);
-    st_sector(a.sink.rows + (u64)id * ROW_WORDS, w0, (u64)succ[0] | ((u64)succ[1] << 32), (u64)succ[2] | ((u64)pred[0] << 32),
-              (u64)pred[1] | ((u64)pred[2] << 32));
-    if (n_out == 4 || n == 4) {
+    const u64 w0 = a.keys[i] | ((u64)(cnt > CNT_CAP ? CNT_CAP : cnt) << 40) | ((u64)e.n_out << 56) | ((u64)e.n_in << 59);
+    st_sector(a.sink.rows + (u64)id * ROW_WORDS, w0, (u64)e.succ[0] | ((u64)e.succ[1] << 32), (u64)e.succ[2] | ((u64)e.pred[0] << 32),
+              (u64)e.pred[1] | ((u64)e.pred[2] << 32));
+    if (e.n_out == 4 || e.n_in == 4) {
         const u32 at = atomicAdd_system(a.sink.n_over, 1u);
-        a.sink.over[at] = make_ulonglong2((u64)id | ((u64)succ[3] << 32), (u64)pred[3]);
+        a.sink.over[at] = make_ulonglong2((u64)id | ((u64)e.succ[3] << 32), (u64)e.pred[3]);
     }
     if (a.sink.kmers) a.sink.kmers[id] = make_ulonglong2(lo, hi);
 }
@@ -2357,9 +2353,9 @@ k_query(QueryArgs a, Geom g, Part pt) {
         for (int b = 0; b < BATCH; b++) {
             if (!live[b]) continue;
             bool hit = k0[b] == lo[b] && k1[b] == hi[b];
-            if (!hit && ((u32)q2[b] & CNT2_DISP)) {   /* (an empty home has no mark) */
+            if (!hit && home_displaced(q2[b])) {
                 const u64 from = idx[b] + 1 == a.cap ? 0 : idx[b] + 1;
-                hit = t2_probe_from(a.table, a.cap, from, lo[b], hi[b], q2[b], q3[b], false) != INF64;
+                hit = t2_probe_from(a.table, a.cap, from, lo[b], hi[b], q2[b], false) != INF64;
             }
             if (hit) { rank[b] = (u32)(q2[b] >> 32); n_found++; }
         }

@@ -283,6 +283,7 @@ struct Shard {
     uint64_t surv_done = 0;                       /* survivor records of the finished rounds (in d_rec) */
     float acc[6] = {};                            /* scatter, init1, pass1, prune, table2, pass2 ms summed over the rounds */
     bool merged() const { return G > 1 || S > 1; } /* the finish builds a table over survivor RECORDS */
+    bool mine(int u) const { return owner[u] == rank && round_of[u] == rnd; } /* unit u is processed here, this round */
     uint64_t bar_seq = 0;                         /* device barriers of this build so far (k_peer_barrier) */
 };
 
@@ -1141,7 +1142,7 @@ int run_passes(vdjgraph_ctx *c) {
         /* table-1 slices of this device's units of this round, in unit order */
         cap1 = 0;
         for (int u = 0; u < sh.NU; u++) {
-            if (sh.owner[u] != sh.rank || sh.round_of[u] != sh.rnd) continue;
+            if (!sh.mine(u)) continue;
             const uint64_t len = unit_slots1(sh, c->prm, u);
             if (cap1 + len > 0xFFFFFFF0ull) return fail(VDJGRAPH_ERR_TOO_MANY_NODES, "pass-1 table would need more than 2^32 slots");
             sh.utab[u].off1 = (u32)cap1; sh.utab[u].len1 = (u32)len;
@@ -1153,7 +1154,7 @@ int run_passes(vdjgraph_ctx *c) {
         uint64_t warps = (uint64_t)grid_p1 * WARPS;
         /* (distinct k-mers, estimated: 1.3x the HyperLogLog figure of this device's units; an overrun doubles it) */
         double est_own = 0;
-        for (int u = 0; u < sh.NU; u++) if (sh.owner[u] == sh.rank && sh.round_of[u] == sh.rnd) est_own += sh.est[u];
+        for (int u = 0; u < sh.NU; u++) if (sh.mine(u)) est_own += sh.est[u];
         const uint64_t distinct_cap = std::min<uint64_t>(std::min<uint64_t>(n_gated, cap1), (uint64_t)(est_own * 1.3) + 4096);
         uint64_t log_cap = (uint64_t)((double)distinct_cap * log_scale) + warps * LOG_CHUNK + LOG_CHUNK;
         if (NB == 0) log_cap = 1;
@@ -1212,9 +1213,9 @@ int run_passes(vdjgraph_ctx *c) {
     uint64_t cap2 = 0;
     {
         double est_own = 0;
-        for (int u = 0; u < sh.NU; u++) if (sh.owner[u] == sh.rank && sh.round_of[u] == sh.rnd) est_own += sh.est[u] + 1.0;
+        for (int u = 0; u < sh.NU; u++) if (sh.mine(u)) est_own += sh.est[u] + 1.0;
         for (int u = 0; u < sh.NU; u++) {
-            if (sh.owner[u] != sh.rank || sh.round_of[u] != sh.rnd) continue;
+            if (!sh.mine(u)) continue;
             const uint64_t len = (uint64_t)((double)n_surv / load2 * (sh.est[u] + 1.0) / est_own) + 64;
             if (cap2 + len > 0x7FFFFFF0ull) return fail(VDJGRAPH_ERR_TOO_MANY_NODES, "survivor table too large");
             sh.utab[u].off2 = (u32)cap2; sh.utab[u].len2 = (u32)len;
@@ -1243,8 +1244,8 @@ int run_passes(vdjgraph_ctx *c) {
     CK(cudaGetLastError());
     res.table1_slots = cap1; res.table2_slots = cap2;
     if (sh.merged()) {
-        /* the survivors as dense records: appended to those of the earlier rounds, ready to be sent
-         * to the finishing device */
+        /* the survivors as dense records, appended to those of the earlier rounds: the finish builds this
+         * device's flat table from them */
         const uint64_t done = sh.surv_done;
         const uint64_t expect = sh.rnd == 0 && sh.S > 1 ? n_surv * (uint64_t)sh.S + n_surv / 8 : done + n_surv;
         if ((rc = c->d_rec.ensure_keep(std::max<uint64_t>(done + n_surv, 1) * sizeof(Slot2), done * sizeof(Slot2), s))) return rc;
@@ -1320,6 +1321,31 @@ int run_hashmap_layout(vdjgraph_ctx *c, uint64_t n) {
     return 0;
 }
 
+/* the finish's flat survivor table (one slice: k-mers are found by slot hash alone) over this device's n survivor
+ * records; pt is set up for the kernels that read it.  Also restarts the node count, which k_compact_table2 used. */
+int table2_from_records(vdjgraph_ctx *c, Part &pt, Slot2 *table, uint64_t cap, uint64_t n) {
+    cudaStream_t s = c->stream;
+    Counters *d_ctr = c->d_ctr.as<Counters>();
+    pt.flat = 1; pt.flat_len = (u32)cap;
+    CK(cudaMemsetAsync(&d_ctr->n_nodes, 0, sizeof(u64), s));
+    k_init_table2<<<c->sm_count * 8, THREADS, 0, s>>>(table, cap);
+    if (n) k_table2_from_records<<<c->sm_count * 8, THREADS, 0, s>>>(c->d_rec.as<Slot2>(), n, table, cap, c->g, pt, d_ctr);
+    c->res.kernel_launches += n ? 2 : 1;
+    return 0;
+}
+
+/* (first_any, slot) of the n nodes of table, sorted by first_any into keys (slots into d_vals[1]).  Allocates nothing:
+ * d_keys[0], d_vals[0..1] and d_cub are sized by the caller (in a sharded build, before the finish's steps are queued). */
+int collect_sorted(vdjgraph_ctx *c, const Slot2 *table, uint64_t cap, uint64_t n, u64 *keys) {
+    cudaStream_t s = c->stream;
+    k_collect<<<c->sm_count * 8, THREADS, 0, s>>>(table, cap, c->d_keys[0].as<u64>(), c->d_vals[0].as<u32>(), c->d_ctr.as<Counters>());
+    c->res.kernel_launches++;
+    size_t cub_bytes = c->d_cub.cap;
+    CK(cub::DeviceRadixSort::SortPairs(c->d_cub.p, cub_bytes, c->d_keys[0].as<u64>(), keys, c->d_vals[0].as<u32>(), c->d_vals[1].as<u32>(),
+                                       (int64_t)n, 0, bits_for(c->sh.total_records * (uint64_t)c->g.w), s));
+    return 0;
+}
+
 /* K5: creation ranks and edge lists on ONE device: straight from its survivor table, or (several rounds) from
  * one table over the survivor records of all rounds.  Several devices: finish_step / finish_end below. */
 int run_finish(vdjgraph_ctx *c) {
@@ -1328,19 +1354,15 @@ int run_finish(vdjgraph_ctx *c) {
     cudaStream_t s = c->stream;
     int rc;
     vdjgraph_result &res = c->res;
-    Counters *d_ctr = c->d_ctr.as<Counters>();
     Counters *h_ctr = c->h_ctr.as<Counters>();
-    const int grid_flat = c->sm_count * 8;
     Part pt = c->part;
     uint64_t n_surv = sh.surv_all[sh.rank];
     uint64_t cap2 = c->cap2;
     Slot2 *table = c->d_t2.as<Slot2>();
     CK(cudaEventRecord(c->ev[EV_FINISH], s));
     if (sh.merged()) {
-        /* several rounds on one device: the survivor records of all rounds */
-        const Slot2 *records = c->d_rec.as<Slot2>();
+        /* several rounds on one device: one table over the survivor records of all rounds */
         n_surv = sh.surv_done;
-        /* merged table: one flat slice (the finish looks k-mers up by slot hash alone) */
         cap2 = std::max<uint64_t>(1024, (uint64_t)((double)n_surv * MERGED_SLOTS_PER_NODE) + 64);
         /* VDJGRAPH_FREE_TABLES_MB = m: when the merged table exceeds m MB, the tables and the log of the last
          * round (dead: the survivors are records now) are freed before the finish takes its own memory, and
@@ -1351,13 +1373,9 @@ int run_finish(vdjgraph_ctx *c) {
             CK(cudaStreamSynchronize(s));
             c->d_t1.release(); c->d_surv.release(); c->d_log.release(); c->d_t2.release();
         }
-        pt.flat = 1; pt.flat_len = (u32)cap2;
         if ((rc = c->d_t2m.ensure(cap2 * sizeof(Slot2)))) return rc;
         table = c->d_t2m.as<Slot2>();
-        CK(cudaMemsetAsync(&d_ctr->n_nodes, 0, sizeof(u64), s));
-        k_init_table2<<<grid_flat, THREADS, 0, s>>>(table, cap2);
-        k_table2_from_records<<<grid_flat, THREADS, 0, s>>>(records, n_surv, table, cap2, g, pt, d_ctr);
-        res.kernel_launches += 2;
+        if ((rc = table2_from_records(c, pt, table, cap2, n_surv))) return rc;
     }
     const size_t na = std::max<uint64_t>(n_surv, 1);
     const bool keys = want_keys(c->prm.flags);
@@ -1365,21 +1383,18 @@ int run_finish(vdjgraph_ctx *c) {
         (rc = c->d_vals[0].ensure(na * 4)) || (rc = c->d_vals[1].ensure(na * 4)) ||
         (rc = c->nodes.ensure(n_surv, keys)))
         return rc;
-    const int end_bit = bits_for(sh.total_records * (uint64_t)g.w);
     size_t cub_bytes = 0;
-    CK(cub::DeviceRadixSort::SortPairs(nullptr, cub_bytes, c->d_keys[0].as<u64>(), c->d_keys[1].as<u64>(),
-                                       c->d_vals[0].as<u32>(), c->d_vals[1].as<u32>(), (int64_t)n_surv, 0, end_bit, s));
+    CK(cub::DeviceRadixSort::SortPairs(nullptr, cub_bytes, c->d_keys[0].as<u64>(), c->d_keys[1].as<u64>(), c->d_vals[0].as<u32>(),
+                                       c->d_vals[1].as<u32>(), (int64_t)n_surv, 0, bits_for(sh.total_records * (uint64_t)g.w), s));
     if ((rc = c->d_cub.ensure(std::max<size_t>(cub_bytes, 16)))) return rc;
     if (n_surv) {
-        k_collect<<<grid_flat, THREADS, 0, s>>>(table, cap2, c->d_keys[0].as<u64>(), c->d_vals[0].as<u32>(), d_ctr);
-        CK(cub::DeviceRadixSort::SortPairs(c->d_cub.p, cub_bytes, c->d_keys[0].as<u64>(), c->d_keys[1].as<u64>(),
-                                           c->d_vals[0].as<u32>(), c->d_vals[1].as<u32>(), (int64_t)n_surv, 0, end_bit, s));
+        if ((rc = collect_sorted(c, table, cap2, n_surv, c->d_keys[1].as<u64>()))) return rc;
         const int gb = (int)((n_surv + THREADS - 1) / THREADS);
         k_assign_rank<<<gb, THREADS, 0, s>>>(table, c->d_vals[1].as<u32>(), n_surv);
         ExportArgs ae = c->nodes.export_args(keys);
         ae.table = table; ae.cap = cap2; ae.keys = c->d_keys[1].as<u64>(); ae.vals = c->d_vals[1].as<u32>(); ae.n = n_surv;
         k_export<<<gb, THREADS, 0, s>>>(ae, g, pt);
-        res.kernel_launches += 3;
+        res.kernel_launches += 2;
     }
     res.hm_buckets = 0; res.ms_hashmap = 0;
     if ((c->prm.flags & VDJGRAPH_FLAG_HASHMAP_LAYOUT) && (rc = run_hashmap_layout(c, n_surv))) return rc;
@@ -1476,26 +1491,14 @@ int finish_step(vdjgraph_ctx *c, int step, bool device_barrier) {
     const uint64_t n_r = sh.surv_all[sh.rank];
     Slot2 *table = reinterpret_cast<Slot2 *>(arena + f.table_off);
     u64 *all_keys = reinterpret_cast<u64 *>(arena + f.keys_off);
-    const int grid_flat = c->sm_count * 8;
     const int gb = (int)std::max<uint64_t>(1, (n_r + THREADS - 1) / THREADS);
     for (int d = 0; d < sh.G; d++)
         if (!sh.peer[d][BUF_GATHER]) return fail(VDJGRAPH_ERR_STATE, "device %d's exchange buffer is not set", d);
     if (step == 0) {
         CK(cudaEventRecord(c->ev[EV_FINISH], s));
         Part pt = c->part;
-        pt.flat = 1; pt.flat_len = (u32)f.cap;
-        CK(cudaMemsetAsync(&d_ctr->n_nodes, 0, sizeof(u64), s));
-        k_init_table2<<<grid_flat, THREADS, 0, s>>>(table, f.cap);
-        res.kernel_launches++;
-        if (n_r) {
-            k_table2_from_records<<<grid_flat, THREADS, 0, s>>>(c->d_rec.as<Slot2>(), n_r, table, f.cap, g, pt, d_ctr);
-            k_collect<<<grid_flat, THREADS, 0, s>>>(table, f.cap, c->d_keys[0].as<u64>(), c->d_vals[0].as<u32>(), d_ctr);
-            size_t cub_bytes = c->d_cub.cap;
-            CK(cub::DeviceRadixSort::SortPairs(c->d_cub.p, cub_bytes, c->d_keys[0].as<u64>(), all_keys + sh.surv_off[sh.rank],
-                                               c->d_vals[0].as<u32>(), c->d_vals[1].as<u32>(), (int64_t)n_r, 0,
-                                               bits_for(sh.total_records * (uint64_t)g.w), s));
-            res.kernel_launches += 2;
-        }
+        if (int rc = table2_from_records(c, pt, table, f.cap, n_r)) return rc;
+        if (int rc = n_r ? collect_sorted(c, table, f.cap, n_r, all_keys + sh.surv_off[sh.rank]) : 0) return rc;
     } else if (step == 1) {
         KeySegs ks;
         for (int d = 0; d <= sh.G; d++) ks.off[d] = sh.surv_off[d];
